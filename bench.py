@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the batched inverse-dynamics hot path (BASELINE.json metric: RNEA samples/s, % of HBM roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype f64|f32] [--samples B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype f64|f32] [--samples B] [--dump-outputs DIR]
     python bench.py --impl reference ...        # the reference's CPU algorithm (oracle port) on the host cores
 
 A "step" is one pass of the fused RNEA kernel over one resident batch of B synthetic (q, qd, qdd) samples
@@ -235,7 +235,11 @@ class RneaWorkload:
     def step(self):
         q, qd, qdd, tau = self.sets[self.k % self.nset]
         self.k += 1
-        self.model.rnea(q, qd, qdd, tau=tau)
+        self.tau = self.model.rnea(q, qd, qdd, tau=tau)
+
+    def outputs(self):
+        """what the last step() returned to its caller: name -> (tensor, axis that runs over the samples)"""
+        return {"tau": (self.tau, 1)}
 
     def e2e_step(self):
         self.model.rnea_host_soa(*self.soa_pinned, tau=self.tau_host_soa)
@@ -303,6 +307,9 @@ class GramWorkload:
         self.model.regressor_gram(q, qd, qdd, f, pack=self.pack)
         self.reducer(self.pack)
 
+    def outputs(self):
+        return {"pack": (self.pack, None)}
+
     def local_step(self):
         """the same without the collective"""
         q, qd, qdd, f = self.sets[self.k % self.nset]
@@ -363,6 +370,9 @@ class LinearizeWorkload:
 
     def step(self):
         self.out = self.model.linearize(self.q, self.qd, None, dt=0.002, eps=1e-8, centered=True)
+
+    def outputs(self):
+        return {"A": (self.out[0], 0), "B": (self.out[1], 0)}
 
     def e2e_step(self):
         q, qd = self.qh.cuda(non_blocking=True), self.qdh.cuda(non_blocking=True)
@@ -475,6 +485,37 @@ def roofline_block(wl, kern_ms_avg, kern_ms_isolated, traffic):
             # the kernel does not load rows its result cannot depend on (rbm_model_live_inputs): `frac` is on SURVEY 8(d)'s contract
             # bytes, `frac_moved` on the bytes the launch really moves through DRAM
             "bytes_moved_per_launch": wl.moved_bytes, "achieved_moved": moved, "frac_moved": moved / peak, "live_input_rows": wl.live_rows}
+
+
+DUMP_BYTES = 64 << 20
+
+
+def sample_outputs(outputs):
+    """Device copies of a step's outputs (name -> (tensor, sample axis or None)), at most DUMP_BYTES in all.  When the outputs are
+    larger, every output that runs over the samples keeps the same sorted subset of them, drawn with a fixed seed, so two runs with
+    the same arguments keep the same samples.  Returns the copies and the number of samples kept (None = all)."""
+    import torch
+
+    nbytes = lambda t: t.numel() * t.element_size()
+    total = sum(nbytes(t) for t, _ in outputs.values())
+    keep = None
+    if total > DUMP_BYTES:
+        (n,) = {t.shape[ax] for t, ax in outputs.values() if ax is not None}
+        fixed = sum(nbytes(t) for t, ax in outputs.values() if ax is None)
+        k = int((DUMP_BYTES - fixed) // ((total - fixed) / n))
+        keep = np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    out = {}
+    for name, (t, ax) in outputs.items():
+        if keep is not None and ax is not None:
+            t = t.index_select(ax, torch.as_tensor(keep, device=t.device))
+        out[name] = t.clone()
+    return out, None if keep is None else len(keep)
+
+
+def write_outputs(dirname, outputs):
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(dirname, f"{name}.npy"), t.cpu().numpy())
 
 
 def traffic_entry(key):
@@ -640,20 +681,30 @@ def run_gpu_arm(args):
     tm.barrier()
     n_heat = tm.heat_count(wl.step, 0.3)  # ~0.3 s of untimed steps so that the clock sampler sees loaded clocks
     tm.barrier()
-    # the K timed steps as one CUDA graph (workloads whose step contains a collective stay eager); every rank decides alike
+    # the K timed steps as one CUDA graph (workloads whose step contains a collective stay eager); every rank decides alike.  In both
+    # launch modes they start at input set 0, so the inputs of the last one depend on the arguments alone (the number of heat steps
+    # before an eager pass comes from a timing estimate)
     graph = None
     if not args.eager and getattr(wl, "graphable", True):
+        wl.k = 0
         graph = tm.capture(wl.step, args.steps)
         (ok,) = tm.max_over_ranks([0.0 if graph is not None else 1.0])
         if ok != 0.0:
             graph = None
+    graph_outputs = wl.outputs() if graph is not None else None  # the buffers the graph's last captured step writes
+    dump = None
     with ClockSampler(local) as clk:
         for _ in range(n_heat):
             wl.step()
+        wl.k = 0
         # pass 1 -- the reported value: exactly K steps back to back, bracketed by barrier + synchronize
         total_ms = tm.timed(wl.step, args.steps, graph=graph)
+        if args.dump_outputs and rank == 0:  # copied before pass 2 runs more steps into the same buffers
+            dump = sample_outputs(graph_outputs or wl.outputs())
         # pass 2 -- per-launch durations (an event pair around every launch, same stream)
         kern_ms_isolated = tm.isolated(wl.step, args.steps)
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump[0])
     # one step == one launch of the dominant kernel (plus, for the Gram workload, a single-CTA finalisation): its average
     # launch duration over the timed region is total / K.  The isolated figure (event pair around every launch) additionally
     # contains the stream bubbles that event records insert between launches and is reported for reference.
@@ -708,6 +759,9 @@ def run_gpu_arm(args):
         }
         if extra:
             line["extra"] = extra
+        if dump is not None:
+            line["outputs"] = {"dir": args.dump_outputs, "arrays": {k: list(t.shape) for k, t in dump[0].items()},
+                               "samples_kept": dump[1] if dump[1] is not None else "all"}
         if world == 1 and not args.no_cpu and args.workload == "rnea":
             if numa.get("bound"):  # the CPU leg forks one worker per host core: undo the socket-local CPU binding first
                 from rigid_body_manipulation_b200 import numa as rbm_numa
@@ -741,7 +795,14 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the extra.* legs (configs[2] Gram + all-reduce, configs[3] linearisation, fp32 RNEA)")
     ap.add_argument("--no-numa", action="store_true", help="do not bind the rank to the GPU's NUMA node")
     ap.add_argument("--gram-samples", type=int, default=12_500_000, help="samples per GPU of the extra.gram leg (12.5 M x 8 GPUs = configs[2]'s 100 M)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (rank 0's shard; at most 64 MB in all, larger outputs "
+                         "keep a fixed seeded subset of the samples), so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

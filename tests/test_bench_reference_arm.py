@@ -31,6 +31,14 @@ def test_reference_arm_prints_one_contract_line_without_a_gpu():
     assert "workload" in d["config"] and "model" not in d["config"]
 
 
+def test_bench_rejects_zero_steps_and_a_dump_of_the_reference_arm(tmp_path):
+    for extra in (("--steps", "0"), ("--dump-outputs", str(tmp_path))):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", *extra], capture_output=True, text=True,
+                             timeout=600, cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+        assert out.returncode == 2 and extra[0] in out.stderr, out.stderr[-2000:]
+        assert not [ln for ln in out.stdout.splitlines() if ln.startswith("{")]
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     out = run({"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2", "CUDA_VISIBLE_DEVICES": ""}, "--gpus", "2")
     assert out.returncode == 0, out.stderr[-2000:]

@@ -72,6 +72,38 @@ def test_other_workloads(extra):
     assert 0 < d["roofline"]["frac"] < 2
 
 
+def test_dump_outputs(tmp_path):
+    """--dump-outputs writes what the last timed step returned: the same in graph-replay and eager mode, equal to the oracle on that
+    step's inputs, identical from run to run, and cut to a seeded subset of the samples when the outputs exceed 64 MB."""
+    import numpy as np
+
+    import bench
+    from oracle import rnea_vec as rv
+
+    n = 262144
+    common = ("--steps", "1", "--warmup", "2", "--no-cpu", "--no-extra", "--samples", str(n))
+    d = run_bench(*common, "--dump-outputs", str(tmp_path / "graph"))
+    assert d["steps"] == 1 and d["config"]["launch_mode"].startswith("CUDA graph") and d["outputs"]["samples_kept"] == "all"
+    run_bench(*common, "--eager", "--dump-outputs", str(tmp_path / "eager"))
+    tau = np.load(tmp_path / "graph" / "tau.npy")
+    assert tau.dtype == np.float64 and tau.shape == (6, n)
+    assert np.array_equal(tau, np.load(tmp_path / "eager" / "tau.npy"))
+    traj = bench.sample_states(np.random.default_rng(1000), n)[::997]  # the first input set is the one the single timed step reads
+    c = bench.load_constants()
+    ref = rv.inverse_batched(traj, c.hposes_Rt, c.simats, c.uscrews, c.twist_0, c.dtwist_0)["tau"]
+    assert np.abs(tau[:, ::997].T - ref).max() < 1e-9 * np.abs(ref).max()
+
+    lin = ("--workload", "linearize", "--samples", "65536", "--steps", "2", "--warmup", "1", "--no-cpu", "--no-extra")  # 113 MB of A, B
+    d = run_bench(*lin, "--dump-outputs", str(tmp_path / "lin1"))
+    run_bench(*lin, "--dump-outputs", str(tmp_path / "lin2"))
+    k = d["outputs"]["samples_kept"]
+    assert 0 < k < 65536
+    for name, shape in (("A", (k, 12, 12)), ("B", (k, 12, 6))):
+        a, b = np.load(tmp_path / "lin1" / f"{name}.npy"), np.load(tmp_path / "lin2" / f"{name}.npy")
+        assert a.shape == shape and a.dtype == np.float64 and np.isfinite(a).all() and np.array_equal(a, b)
+    assert sum(os.path.getsize(tmp_path / "lin1" / f) for f in os.listdir(tmp_path / "lin1")) <= bench.DUMP_BYTES + 1024
+
+
 def test_reference_arm_line():
     d = run_bench("--impl", "reference", "--steps", "2", "--warmup", "1", "--cpu-samples", "128")
     check_common(d)

@@ -143,22 +143,19 @@ def test_tau_is_affine_in_qdd():
     assert np.allclose(t3 - t2, t2 - t0, atol=1e-10)
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not rl.available(), reason="reference checkout absent (GPU box)")
 def test_oracle_matches_reference_files_live():
-    ns = rl.load()
-    g = load_golden("ref_inverse_hammer.npz")
-    rng = np.random.default_rng(12345)
-    hp_ref = [ns.liegroups.SE3(ns.liegroups.SO3(r[:9].reshape(3, 3).copy()), r[9:].copy()) for r in g["hposes_Rt"]]
-    hp_or = [se3_from_Rt(r) for r in g["hposes_Rt"]]
-    for _ in range(20):
-        traj = np.stack([rng.uniform(-7, 7, 6), rng.standard_normal(6), rng.standard_normal(6) * 4])
-        a = ns.dynamics.inverse(traj, hp_ref, g["simats"], g["uscrews"], g["twist_0"], g["dtwist_0"])
-        b = ro.inverse(traj, hp_or, g["simats"], g["uscrews"], g["twist_0"], g["dtwist_0"])
-        assert np.allclose(a[0], b[0], rtol=1e-14, atol=1e-13)
-        assert np.allclose(np.array(a[2]), np.array(b[2]), atol=1e-14)
-        assert np.allclose(np.array(a[3]), np.array(b[3]), rtol=1e-14, atol=1e-13)
-        assert np.allclose(ns.dynamics.get_regressor_matrix(a[2][6], a[3][6]), ro.regressor(b[2][6], b[3][6]), atol=1e-13)
+    """Every stored sample of the reference's own dynamics.inverse (oracle/gen_golden.py) against the per-sample oracle, at the
+    tolerances of a side-by-side run of the two."""
+    for t in TARGETS:
+        g = load_golden(f"ref_inverse_{t}.npz")
+        hp = [se3_from_Rt(r) for r in g["hposes_Rt"]]
+        pose_sen = se3_from_Rt(g["pose_sen_llj"])
+        for s, traj in enumerate(g["traj"]):
+            tau, _, tw, dtw = ro.inverse(traj, hp, g["simats"], g["uscrews"], g["twist_0"], g["dtwist_0"])
+            assert np.allclose(tau, g["tau"][s], rtol=1e-14, atol=1e-13)
+            assert np.allclose(np.array(tw), g["twists"][s], atol=1e-14)
+            assert np.allclose(np.array(dtw), g["dtwists"][s], rtol=1e-14, atol=1e-13)
+            assert np.allclose(ro.regressor(*ro.sensor_frame_twists(pose_sen, tw[-1], dtw[-1])), g["regressor"][s], atol=1e-13)
 
 
 @pytest.mark.reference

@@ -1,11 +1,11 @@
-"""The closed-loop path pinned to THE REFERENCE'S OWN CODE: core/simulate.py::simulate, controllers/lqr.py, the planner, sensors and pose
-registers are executed unmodified from /root/reference on the functional MuJoCo stand-in (oracle/mujoco_standin.py).
+"""The closed-loop path pinned to THE REFERENCE'S OWN CODE: tests/golden/ref_simulate_{hammer,uniform_gearbox}.npz hold what the
+reference's core/simulate.py::simulate returned (controllers/lqr.py, the planner, sensors and pose registers executed unmodified on the
+functional MuJoCo stand-in of oracle/mujoco_standin.py, full 1500-step runs written by oracle/gen_golden_simulate.py).
 
-  * live (needs the checkout; skipped on the GPU box): a short run of the reference's simulate() == oracle/replay_oracle.py, i.e. the
-    restated loop (frame schedule, lagged qacc / sensordata, control law, sensor-frame twists, noise model) is the reference's;
-  * golden (tests/golden/ref_simulate_hammer.npz, written by oracle/gen_golden_simulate.py from the full 1500-step reference run): the
-    kernels' rollout algorithm (host build of csrc/rbm_dynamics.cuh here, the CUDA kernel in tests/test_gpu_replay.py) reproduces what the
-    reference's simulate() returned.
+  * oracle/replay_oracle.py reproduces those runs, i.e. the restated loop (LQR gain, frame schedule, lagged qacc / sensordata, control
+    law, sensor-frame twists, noise model) is the reference's;
+  * the kernels' rollout algorithm (host build of csrc/rbm_dynamics.cuh here, the CUDA kernel in tests/test_gpu_replay.py) reproduces
+    them too.
 What the stand-in restates of MuJoCo (plant step, F/T sensor) is listed in its header; that part stays unpinned against MuJoCo itself."""
 import os
 
@@ -13,7 +13,6 @@ import numpy as np
 import pytest
 
 from conftest import load_golden
-from oracle import reference_loader as rl
 from oracle import replay_oracle as ro
 from oracle import rnea_vec as rv
 from rigid_body_manipulation_b200 import engine, identification as idn, planner
@@ -25,22 +24,17 @@ def _consts(g):
     return dict(hposes_Rt=g["hposes_Rt"], simats=g["simats"], uscrews=g["uscrews"], twist_0=g["twist_0"], dtwist_0=g["dtwist_0"])
 
 
-@pytest.mark.skipif(not rl.available(), reason="reference checkout not present")
 def test_reference_simulate_equals_the_restated_loop():
-    from oracle.gen_golden_simulate import run_reference_simulation
-
-    res, controller, pl, m = run_reference_simulation("kill_la_kill", duration=0.5)        # 250 steps, 25 frames
-    K = controller.gain_matrix
-    Kr = ro.lqr_gain(m.consts, m.key_qpos, np.zeros(6), [10.0, 10.0, 10.0, 1e4, 1e4, 1e4])
-    assert np.abs(K - Kr).max() < 1e-12 * np.abs(Kr).max()            # the reference's controller on the stand-in == the restatement
-    plan_traj = np.array([pl.plan(k) for k in range(pl.n_steps)])
-    out = ro.closed_loop_replay(m.consts, m.pose_sen_Rt, m.G_sensed, plan_traj, K, m.key_qpos)
-    fr = res["frames"]
-    assert len(fr) == len(out["step"]) == 25
-    for key, mine in (("twist_sen", out["twist_sen"]), ("dtwist_sen", out["dtwist_sen"]), ("ft_sen", idn.perturb_wrench(out["wrench"], 0.05, 0))):
-        theirs = np.array([f[key] for f in fr])
-        assert np.abs(theirs - mine).max() < 1e-12 * np.abs(mine).max(), key
-    assert np.abs(np.asarray(res["regressors"]) - out["regressor"]).max() < 1e-12 * np.abs(out["regressor"]).max()
+    for target in ("hammer", "uniform_gearbox"):
+        g = load_golden(f"ref_simulate_{target}.npz")
+        Kr = ro.lqr_gain(_consts(g), g["key_qpos"], np.zeros(6), [10.0, 10.0, 10.0, 1e4, 1e4, 1e4])
+        assert np.abs(g["gain_matrix"] - Kr).max() < 1e-12 * np.abs(Kr).max()    # the reference's controller on the stand-in == the restatement
+        pl = planner.QuinticPlan(g["displacements"], g["key_qpos"], float(g["timestep"]), int(g["n_steps"]))
+        out = ro.closed_loop_replay(_consts(g), g["pose_sen_llj"], g["G_sensed"], pl.trajectory(), Kr, g["key_qpos"])
+        assert len(out["step"]) == g["twist_sen"].shape[0] == 150
+        for key, mine in (("twist_sen", out["twist_sen"]), ("dtwist_sen", out["dtwist_sen"]), ("ft_sen", idn.perturb_wrench(out["wrench"], 0.05, 0))):
+            assert np.abs(g[key] - mine).max() < 1e-12 * np.abs(mine).max(), (target, key)
+        assert np.abs(g["regressors"] - out["regressor"]).max() < 1e-12 * np.abs(out["regressor"]).max(), target
 
 
 @pytest.mark.parametrize("target", ["hammer", "uniform_gearbox"])
