@@ -99,7 +99,9 @@ RBM_API int rbm_model_kernel_path(const rbm_model* m);
  * Batched dynamics.inverse (dynamics/dynamics.py:109-157): tau[j][s] for every sample s.
  *   q, qd, qdd : [nj][ld]   tau : [nj][ld]
  *   twist_last, dtwist_last : [6][ld] or NULL -- V and dV of the last link (twists[nj], dtwists[nj] of
- *   the reference's return value; the only entries core/simulate.py:203,206 reads). */
+ *   the reference's return value; the only entries core/simulate.py:203,206 reads).
+ * On a fast-path model the kernels never read the gantry positions q[0..2], and a call without twists does not read the gantry
+ * velocities qd[0..2] either (tau does not depend on them): the caller may leave those rows unset. */
 RBM_API int rbm_rnea_f64(const rbm_model* m, const double* q, const double* qd, const double* qdd, double* tau, double* twist_last,
                  double* dtwist_last, int64_t n, int64_t ld, void* stream);
 RBM_API int rbm_rnea_f32(const rbm_model* m, const float* q, const float* qd, const float* qdd, float* tau, float* twist_last,
@@ -138,15 +140,18 @@ RBM_API int rbm_rnea_planned_f32(const rbm_model* m, const double* coeffs, const
 RBM_API int rbm_rnea_host_f64(const rbm_model* m, const double* traj_host, double* tau_host, int64_t n, int64_t chunk);
 RBM_API int rbm_rnea_host_f32(const rbm_model* m, const float* traj_host, float* tau_host, int64_t n, int64_t chunk);
 
-/* Which rows of (q, qd, qdd) the model's inverse-dynamics kernels read: mask [3][nj], 1 = live, 0 = the result does not depend on
- * it and the kernel never loads it.  For the reference's structure (three leading prismatic joints, core/simulate.py:98-110,
- * xml_models/manipulators/sequential.xml:13-39) tau, V_6 and dV_6 do not depend on the gantry positions q_0..q_2, so 15 of the
- * 18 input rows are live: 168 instead of 192 bytes of DRAM traffic per fp64 sample, and 15 rows instead of 18 over PCIe. */
+/* Which rows of (q, qd, qdd) the model's inverse-dynamics kernels read when every output (tau, V_6, dV_6) is asked for: mask [3][nj],
+ * 1 = live, 0 = the result does not depend on it and the kernel never loads it.  For the reference's structure (three leading
+ * prismatic joints, core/simulate.py:98-110, xml_models/manipulators/sequential.xml:13-39) tau, V_6 and dV_6 do not depend on the
+ * gantry positions q_0..q_2, so 15 of the 18 input rows are live.  A tau-only call reads three rows fewer: tau does not depend on
+ * the gantry velocities qd_0..qd_2 either (a Galilean boost, no rotation precedes those joints), so it loads 12 rows -- 144
+ * instead of 192 bytes of DRAM traffic per fp64 sample -- and rbm_rnea_host_soa_* uploads those 12. */
 RBM_API int rbm_model_live_inputs(const rbm_model* m, int32_t* mask);
 
 /* The same end-to-end path for the kernels' own SoA layout (what dynamics.inverse would be handed by a caller that batches a
- * whole trajectory: rows of q, qd, qdd): q_host, qd_host, qdd_host, tau_host are HOST buffers [nj][ld].  Only LIVE rows
- * (rbm_model_live_inputs) are uploaded -- one strided cudaMemcpy2DAsync per run of live rows and chunk -- and tau comes back
+ * whole trajectory: rows of q, qd, qdd): q_host, qd_host, qdd_host, tau_host are HOST buffers [nj][ld].  Only the rows the tau-only
+ * kernel reads are uploaded (on a fast-path model: not q[0..2], not qd[0..2], which the caller may leave unset; see
+ * rbm_model_live_inputs) -- one strided cudaMemcpy2DAsync per run of live rows and chunk -- and tau comes back
  * with one strided copy per chunk, both overlapped with the kernel over three internal streams.  Synchronous. */
 RBM_API int rbm_rnea_host_soa_f64(const rbm_model* m, const double* q_host, const double* qd_host, const double* qdd_host, double* tau_host,
                           int64_t n, int64_t ld, int64_t chunk);

@@ -206,12 +206,15 @@ static int64_t default_chunk(int64_t n) {
   return c;
 }
 
-// which rows of (q, qd, qdd) the inverse-dynamics kernel of this model reads: [3][nj], 1 = live
-static void live_inputs(const rbm_model* m, int32_t* mask) {
+// which rows of (q, qd, qdd) the inverse-dynamics kernel of this model reads: [3][nj], 1 = live.  twists: V_6 / dV_6 are asked for too.
+static void live_inputs(const rbm_model* m, int32_t* mask, bool twists) {
   for (int i = 0; i < 3 * m->nj; ++i) mask[i] = 1;
+  if (m->path == PATH_GENERIC) return;
   // sequential structure (SequentialDesc::q_matters): tau, V_6 and dV_6 do not depend on the three gantry positions
-  if (m->path != PATH_GENERIC)
-    for (int j = 0; j < 3; ++j) mask[j] = 0;
+  for (int j = 0; j < 3; ++j) mask[j] = 0;
+  // SequentialDesc::qd_matters: tau does not depend on the three gantry velocities either (V_6 does)
+  if (!twists)
+    for (int j = 0; j < 3; ++j) mask[m->nj + j] = 0;
 }
 
 // SoA host entry: q, qd, qdd [nj][ld] on the host -> tau [nj][ld] on the host.  Dead rows stay on the host.
@@ -232,7 +235,7 @@ int rnea_host_soa(const rbm_model* m, const T* q_host, const T* qd_host, const T
   constexpr int kSlots = rbm_model::kPipeSlots;
   if (int rc0 = ensure_pipe(m, sizeof(T) * chunk * 3 * nj, sizeof(T) * chunk * nj)) return rc0;
   int32_t live[3 * RBM_MAX_JOINTS];
-  live_inputs(m, live);
+  live_inputs(m, live, false);
   const T* src[3] = {q_host, qd_host, qdd_host};
   int rc = RBM_OK;
   int slot = 0;
@@ -576,7 +579,7 @@ int rbm_rnea_planned_host_f32(const rbm_model* m, const double* coeffs, const do
 }
 int rbm_model_live_inputs(const rbm_model* m, int32_t* mask) {
   if (!m || !mask) return invalid("rbm_model_live_inputs: NULL argument");
-  live_inputs(m, mask);
+  live_inputs(m, mask, true);
   return RBM_OK;
 }
 

@@ -2,7 +2,8 @@
 //
 // One sample per thread; consecutive threads own consecutive samples, so every SoA stream
 // (q_j, qd_j, qdd_j, tau_j) is read / written as fully coalesced 128-byte lines and nothing is
-// re-read: HBM traffic == algorithmic traffic == 24 * sizeof(T) bytes per sample.
+// re-read.  Rows the result does not depend on are not loaded (SoaRows): a tau-only launch on the
+// sequential structure moves 18 * sizeof(T) bytes per sample of the 24 the rows hold.
 #include <atomic>
 #include <cstdlib>
 #include <cstring>
@@ -47,10 +48,18 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), unsigned grid, unsigned 
 // ---------------------------------------------------------------------------------------------
 // fast path, SoA
 // ---------------------------------------------------------------------------------------------
+// Rows of (q, qd, qdd) -- a = 0, 1, 2 -- that the fast SoA kernels load: never the gantry positions, the gantry velocities only when
+// the twist is asked for (SequentialDesc::q_matters / qd_matters).
+template <class D, bool OUT_TWIST>
+struct SoaRows {
+  static constexpr bool live(int a, int j) { return a == 0 ? D::q_matters(j) : a == 1 ? (OUT_TWIST || D::qd_matters(j)) : true; }
+};
+
 template <class T, class D, bool OUT_TWIST>
 __global__ void __launch_bounds__(kBlock) k_rnea_fast_soa(const __grid_constant__ FastParams<T> P, const T* __restrict__ q,
                                                           const T* __restrict__ qd, const T* __restrict__ qdd, T* __restrict__ tau,
                                                           T* __restrict__ Vout, T* __restrict__ dVout, int64_t n, int64_t ld) {
+  using Rows = SoaRows<D, OUT_TWIST>;
   // Programmatic dependent launch: let the next kernel in the stream be scheduled while this grid drains, and wait for
   // the previous grid's memory to be visible before the first global read (stream-order semantics are unchanged).
   pdl_launch_dependents();
@@ -60,12 +69,12 @@ __global__ void __launch_bounds__(kBlock) k_rnea_fast_soa(const __grid_constant_
   T rq[6], rqd[6], rqdd[6];
 #pragma unroll
   for (int j = 0; j < 6; ++j) {
-    rq[j] = __ldg(q + j * ld + s);
-    rqd[j] = __ldg(qd + j * ld + s);
+    rq[j] = Rows::live(0, j) ? __ldg(q + j * ld + s) : T(0);
+    rqd[j] = Rows::live(1, j) ? __ldg(qd + j * ld + s) : T(0);
     rqdd[j] = __ldg(qdd + j * ld + s);
   }
   FastResult<T> r;
-  fast_rnea<T, D, true>(P, rq, rqd, rqdd, r);
+  fast_rnea_tau<T, D, OUT_TWIST>(P, rq, rqd, rqdd, r);
 #pragma unroll
   for (int j = 0; j < 6; ++j) tau[j * ld + s] = r.tau[j];
   if constexpr (OUT_TWIST) {
@@ -85,31 +94,33 @@ template <class D, bool OUT_TWIST>
 __global__ void __launch_bounds__(kBlock) k_rnea_fast_soa_f32x2(const __grid_constant__ FastParams<float> P, const float* __restrict__ q,
                                                                 const float* __restrict__ qd, const float* __restrict__ qdd, float* __restrict__ tau,
                                                                 float* __restrict__ Vout, float* __restrict__ dVout, int64_t n, int64_t ld) {
+  using Rows = SoaRows<D, OUT_TWIST>;
   pdl_launch_dependents();
   pdl_wait_prior_grids();
   const int64_t s = 2 * ((int64_t)blockIdx.x * kBlock + threadIdx.x);
   if (s >= n) return;
   float a_q[6], a_qd[6], a_qdd[6], b_q[6], b_qd[6], b_qdd[6];
   const bool pair = s + 1 < n;
+  const float2 zero = make_float2(0.f, 0.f);
   if (pair) {
 #pragma unroll
     for (int j = 0; j < 6; ++j) {
-      const float2 v0 = __ldg(reinterpret_cast<const float2*>(q + j * ld + s));
-      const float2 v1 = __ldg(reinterpret_cast<const float2*>(qd + j * ld + s));
+      const float2 v0 = Rows::live(0, j) ? __ldg(reinterpret_cast<const float2*>(q + j * ld + s)) : zero;
+      const float2 v1 = Rows::live(1, j) ? __ldg(reinterpret_cast<const float2*>(qd + j * ld + s)) : zero;
       const float2 v2 = __ldg(reinterpret_cast<const float2*>(qdd + j * ld + s));
       a_q[j] = v0.x; b_q[j] = v0.y; a_qd[j] = v1.x; b_qd[j] = v1.y; a_qdd[j] = v2.x; b_qdd[j] = v2.y;
     }
   } else {
 #pragma unroll
     for (int j = 0; j < 6; ++j) {
-      a_q[j] = b_q[j] = __ldg(q + j * ld + s);
-      a_qd[j] = b_qd[j] = __ldg(qd + j * ld + s);
+      a_q[j] = b_q[j] = Rows::live(0, j) ? __ldg(q + j * ld + s) : 0.f;
+      a_qd[j] = b_qd[j] = Rows::live(1, j) ? __ldg(qd + j * ld + s) : 0.f;
       a_qdd[j] = b_qdd[j] = __ldg(qdd + j * ld + s);
     }
   }
   FastResult<float> ra, rb;
-  fast_rnea<float, D, true>(P, a_q, a_qd, a_qdd, ra);
-  fast_rnea<float, D, true>(P, b_q, b_qd, b_qdd, rb);
+  fast_rnea_tau<float, D, OUT_TWIST>(P, a_q, a_qd, a_qdd, ra);
+  fast_rnea_tau<float, D, OUT_TWIST>(P, b_q, b_qd, b_qdd, rb);
   if (pair) {
 #pragma unroll
     for (int j = 0; j < 6; ++j) *reinterpret_cast<float2*>(tau + j * ld + s) = make_float2(ra.tau[j], rb.tau[j]);
@@ -209,7 +220,7 @@ __global__ void __launch_bounds__(kBlock) k_rnea_fast_aos(const __grid_constant_
     T rq[6], rqd[6], rqdd[6];
 #pragma unroll
     for (int j = 0; j < 6; ++j) { rq[j] = my[j]; rqd[j] = my[6 + j]; rqdd[j] = my[12 + j]; }
-    fast_rnea<T, D, true>(P, rq, rqd, rqdd, r);
+    fast_rnea_tau<T, D, false>(P, rq, rqd, rqdd, r);
   }
   __syncthreads();
   if (threadIdx.x < cnt) {
@@ -266,7 +277,7 @@ __global__ void __launch_bounds__(kBlock) k_rnea_fast_aos_tma(const __grid_const
     __syncthreads();                          // inputs are in registers everywhere; out_buf[it & 1] is free
     if (tid == 0) issue(it + S);
     FastResult<T> r;
-    fast_rnea<T, D, true>(P, rq, rqd, rqdd, r);
+    fast_rnea_tau<T, D, false>(P, rq, rqd, rqdd, r);
     T* out = out_buf + (size_t)(it & 1) * kBlock * 6;
 #pragma unroll
     for (int j = 0; j < 6; ++j) out[tid * 6 + j] = r.tau[j];
@@ -287,7 +298,7 @@ __global__ void __launch_bounds__(kBlock) k_rnea_fast_aos_tma(const __grid_const
 #pragma unroll
       for (int j = 0; j < 6; ++j) { rq[j] = __ldg(my + j); rqd[j] = __ldg(my + 6 + j); rqdd[j] = __ldg(my + 12 + j); }
       FastResult<T> r;
-      fast_rnea<T, D, true>(P, rq, rqd, rqdd, r);
+      fast_rnea_tau<T, D, false>(P, rq, rqd, rqdd, r);
 #pragma unroll
       for (int j = 0; j < 6; ++j) tau[s * 6 + j] = r.tau[j];
     }
@@ -333,7 +344,7 @@ __global__ void __launch_bounds__(kBlock) k_rnea_planned_fast(const __grid_const
     rqdd[j] = pl.disp[j] * sa;
   }
   FastResult<T> r;
-  fast_rnea<T, D, true>(P, rq, rqd, rqdd, r);
+  fast_rnea_tau<T, D, false>(P, rq, rqd, rqdd, r);
 #pragma unroll
   for (int j = 0; j < 6; ++j) tau[j * ld + s] = r.tau[j];
   if (traj) {

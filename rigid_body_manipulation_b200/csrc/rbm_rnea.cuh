@@ -179,15 +179,18 @@ RBM_HD void fast_sincos(const T (&q)[6], T (&c)[6], T (&s)[6]) {
   }
 }
 
-template <class T, class D, bool WANT_TAU, bool VEL = true, bool GRAV = true, bool ACC = true, int ONEHOT = -1>
+// TWIST = false: the caller reads tau only, so the joint velocities tau does not depend on (!D::qd_matters) are structural zeros --
+// their loads and their share of the recursion disappear.  FastResult::v/w/a/l are then NOT the physical twist of the last link
+// (they miss the Galilean boost of the gantry velocities).
+template <class T, class D, bool WANT_TAU, bool VEL = true, bool GRAV = true, bool ACC = true, int ONEHOT = -1, bool TWIST = true>
 RBM_HD void fast_rnea_core(const FastParams<T>& P, const T* g, const T (&q)[6], const T (&c)[6], const T (&s)[6], const T (&qd)[6],
                            const T (&qdd)[6], FastResult<T>& out);
 
 // Joint sines / cosines supplied by the caller (the linearisation re-uses them across its many evaluations).
-template <class T, class D, bool WANT_TAU>
+template <class T, class D, bool WANT_TAU, bool TWIST = true>
 RBM_HD void fast_rnea_cs(const FastParams<T>& P, const T (&q)[6], const T (&c)[6], const T (&s)[6], const T (&qd)[6], const T (&qdd)[6],
                          FastResult<T>& out) {
-  fast_rnea_core<T, D, WANT_TAU>(P, P.g, q, c, s, qd, qdd, out);
+  fast_rnea_core<T, D, WANT_TAU, true, true, true, -1, TWIST>(P, P.g, q, c, s, qd, qdd, out);
 }
 
 // Full RNEA for one sample.  WANT_TAU = false leaves the backward sweep out (regressor kernels).
@@ -198,6 +201,17 @@ RBM_HD void fast_rnea(const FastParams<T>& P, const T (&q)[6], const T (&qd)[6],
   fast_rnea_cs<T, D, WANT_TAU>(P, q, c, s, qd, qdd, out);
 }
 
+// What the inverse-dynamics kernels return for one sample: tau from the TWIST = false recursion and, with OUT_TWIST, V_6 / dV_6 from a
+// second forward sweep that keeps every joint velocity.  tau is the same arithmetic whether or not the twist is asked for, so the two
+// forms return the same bits.
+template <class T, class D, bool OUT_TWIST>
+RBM_HD void fast_rnea_tau(const FastParams<T>& P, const T (&q)[6], const T (&qd)[6], const T (&qdd)[6], FastResult<T>& out) {
+  T c[6], s[6];
+  fast_sincos<T, D>(q, c, s);
+  fast_rnea_cs<T, D, true, false>(P, q, c, s, qd, qdd, out);
+  if constexpr (OUT_TWIST) fast_rnea_cs<T, D, false>(P, q, c, s, qd, qdd, out);  // overwrites v/w/a/l only
+}
+
 // The recursion itself; `g` is the linear part of the base acceleration (P.g, or zeros when the joint-space inertia
 // matrix is being extracted column by column).
 // VEL = false treats every joint velocity as a structural zero, GRAV = false the base acceleration and ACC = false every joint
@@ -205,7 +219,7 @@ RBM_HD void fast_rnea(const FastParams<T>& P, const T (&q)[6], const T (&qd)[6],
 // (ACC off, GRAV off) the velocity-product term C(q, qd) alone.  ONEHOT = j >= 0 (with VEL and GRAV off) evaluates qdd = e_j with every
 // other joint acceleration a STRUCTURAL zero: column j of the inertia matrix, where the links before j carry no motion at all and the
 // typed algebra removes their share of the recursion (the linearisation builds M this way: about half the work of six general columns).
-template <class T, class D, bool WANT_TAU, bool VEL, bool GRAV, bool ACC, int ONEHOT>
+template <class T, class D, bool WANT_TAU, bool VEL, bool GRAV, bool ACC, int ONEHOT, bool TWIST>
 RBM_HD void fast_rnea_core(const FastParams<T>& P, const T* g, const T (&q)[6], const T (&c)[6], const T (&s)[6], const T (&qd)[6],
                            const T (&qdd)[6], FastResult<T>& out) {
   // base: twist_0 = 0, dtwist_0 = [g; 0]  (core/simulate.py:149,154-155)
@@ -216,8 +230,8 @@ RBM_HD void fast_rnea_core(const FastParams<T>& P, const T* g, const T (&q)[6], 
     else return Z3{};
   }();
   auto l0 = Z3{};
-  auto vel = [&](int i) {
-    if constexpr (VEL) return qd[i];
+  auto vel = [&](auto I) {
+    if constexpr (VEL && (TWIST || D::qd_matters(decltype(I)::value))) return qd[decltype(I)::value];
     else return Z{};
   };
   auto acc = [&](auto I) {
@@ -228,12 +242,12 @@ RBM_HD void fast_rnea_core(const FastParams<T>& P, const T* g, const T (&q)[6], 
     else return Z{};
   };
   using std::integral_constant;
-  auto k0 = fwd_link<typename D::L0, 0>(P, q[0], vel(0), acc(integral_constant<int, 0>{}), c[0], s[0], v0, w0, a0, l0);
-  auto k1 = fwd_link<typename D::L1, 1>(P, q[1], vel(1), acc(integral_constant<int, 1>{}), c[1], s[1], k0.v, k0.w, k0.a, k0.l);
-  auto k2 = fwd_link<typename D::L2, 2>(P, q[2], vel(2), acc(integral_constant<int, 2>{}), c[2], s[2], k1.v, k1.w, k1.a, k1.l);
-  auto k3 = fwd_link<typename D::L3, 3>(P, q[3], vel(3), acc(integral_constant<int, 3>{}), c[3], s[3], k2.v, k2.w, k2.a, k2.l);
-  auto k4 = fwd_link<typename D::L4, 4>(P, q[4], vel(4), acc(integral_constant<int, 4>{}), c[4], s[4], k3.v, k3.w, k3.a, k3.l);
-  auto k5 = fwd_link<typename D::L5, 5>(P, q[5], vel(5), acc(integral_constant<int, 5>{}), c[5], s[5], k4.v, k4.w, k4.a, k4.l);
+  auto k0 = fwd_link<typename D::L0, 0>(P, q[0], vel(integral_constant<int, 0>{}), acc(integral_constant<int, 0>{}), c[0], s[0], v0, w0, a0, l0);
+  auto k1 = fwd_link<typename D::L1, 1>(P, q[1], vel(integral_constant<int, 1>{}), acc(integral_constant<int, 1>{}), c[1], s[1], k0.v, k0.w, k0.a, k0.l);
+  auto k2 = fwd_link<typename D::L2, 2>(P, q[2], vel(integral_constant<int, 2>{}), acc(integral_constant<int, 2>{}), c[2], s[2], k1.v, k1.w, k1.a, k1.l);
+  auto k3 = fwd_link<typename D::L3, 3>(P, q[3], vel(integral_constant<int, 3>{}), acc(integral_constant<int, 3>{}), c[3], s[3], k2.v, k2.w, k2.a, k2.l);
+  auto k4 = fwd_link<typename D::L4, 4>(P, q[4], vel(integral_constant<int, 4>{}), acc(integral_constant<int, 4>{}), c[4], s[4], k3.v, k3.w, k3.a, k3.l);
+  auto k5 = fwd_link<typename D::L5, 5>(P, q[5], vel(integral_constant<int, 5>{}), acc(integral_constant<int, 5>{}), c[5], s[5], k4.v, k4.w, k4.a, k4.l);
 
   out.v[0] = to_scalar<T>(k5.v.x); out.v[1] = to_scalar<T>(k5.v.y); out.v[2] = to_scalar<T>(k5.v.z);
   out.w[0] = to_scalar<T>(k5.w.x); out.w[1] = to_scalar<T>(k5.w.y); out.w[2] = to_scalar<T>(k5.w.z);

@@ -268,9 +268,10 @@ class Model:
         return tau
 
     def rnea_host_soa(self, q, qd, qdd, tau=None, chunk=0):
-        """SoA host entry: q, qd, qdd HOST buffers (nj, n) -> tau (nj, n) on the host.  Only the rows the model's kernel path
-        actually reads cross the bus (`live_inputs()`: the sequential structure never reads the three gantry positions, so 15 of
-        the 18 input rows are uploaded), one cudaMemcpyAsync per live row and chunk, pipelined with the kernel and the D2H of tau."""
+        """SoA host entry: q, qd, qdd HOST buffers (nj, n) -> tau (nj, n) on the host.  Only the rows the model's tau-only kernel
+        actually reads cross the bus: for the sequential structure neither the three gantry positions (`live_inputs()`) nor the
+        three gantry velocities, which tau does not depend on, so 12 of the 18 input rows are uploaded and the caller may leave
+        q[:3] and qd[:3] unset.  One strided copy per run of live rows and chunk, pipelined with the kernel and the D2H of tau."""
         bufs = []
         for name, a in (("q", q), ("qd", qd), ("qdd", qdd)):
             arr, is_t, dt = self._host_array(a, name)
@@ -314,7 +315,9 @@ class Model:
         return tau
 
     def live_inputs(self):
-        """Boolean mask (3, nj): which rows of (q, qd, qdd) the model's inverse-dynamics kernel reads (rbm_model_live_inputs)."""
+        """Boolean mask (3, nj): which rows of (q, qd, qdd) the model's inverse-dynamics kernel reads when the twists are asked for
+        too (rbm_model_live_inputs).  A tau-only call (`rnea` without want_twists, `rnea_host_soa`) on the sequential structure also
+        skips the three gantry velocities qd[:3]."""
         mask = np.zeros(3 * self.nj, dtype=np.int32)
         rc = self._lib.rbm_model_live_inputs(self._h, _ptr(mask))
         _lib.check(rc, "rbm_model_live_inputs")
