@@ -3,6 +3,7 @@ import numpy as np
 import torch
 
 from conftest import load_golden
+from model_classes import sample_states  # torch-free, shared with the CPU suite
 
 
 def rel_err(a, b, floor=1e-6):
@@ -25,14 +26,6 @@ def soa(traj, dtype=torch.float64):
     """(n, 3, nj) host array -> three contiguous CUDA tensors (nj, n)."""
     t = torch.as_tensor(np.ascontiguousarray(traj), dtype=dtype, device="cuda")
     return tuple(t[:, k, :].t().contiguous() for k in range(3))
-
-
-def sample_states(rng, n):
-    """SURVEY.md 8(d) config-2 input distribution (same as oracle/gen_golden.py)."""
-    q = np.concatenate([rng.uniform(-1.5, 2.5, (n, 3)), rng.uniform(-6 * np.pi, 6 * np.pi, (n, 3))], axis=1)
-    qd = rng.standard_normal((n, 6)) * np.array([1, 1, 1, 3, 3, 3.0])
-    qdd = rng.standard_normal((n, 6)) * np.array([3, 3, 3, 10, 10, 10.0])
-    return np.stack([q, qd, qdd], axis=1)
 
 
 __all__ = ["rel_err", "model_from_golden", "soa", "sample_states", "load_golden"]

@@ -38,25 +38,31 @@ def test_fused_regressor_from_trajectory(fname, force_generic):
     assert rel_err(out["wrench"].t().cpu().numpy(), g["regressor"] @ phi).max() < 1e-9
     # fp32 mode
     q32, qd32, qdd32 = soa(g["traj"], torch.float32)
-    o32 = m.regressor_from_traj(q32, qd32, qdd32)
+    o32 = m.regressor_from_traj(q32, qd32, qdd32, want_rows=True, want_twists=True, phi=phi)
     assert rel_err(o32["Y"].cpu().numpy(), g["regressor"]).max() < 1e-4
+    assert rel_err(o32["twist_sen"].t().cpu().numpy(), g["twist_sen"]).max() < 1e-4
+    assert rel_err(o32["dtwist_sen"].t().cpu().numpy(), g["dtwist_sen"]).max() < 1e-4
+    assert rel_err(o32["wrench"].t().cpu().numpy(), g["regressor"] @ phi).max() < 1e-4
 
 
 @pytest.mark.parametrize("n", [4096, 262_144 + 256 * 5 + 100])
 def test_gram_fp32_mode(n):
-    g = load_golden("ref_inverse_hammer.npz")
+    """The fast model (TMA and direct-load fp32 kernels) and a generic six-joint model (k_regressor_gram<float, PATH_GENERIC>)."""
     rng = np.random.default_rng(n)
     traj = sample_states(rng, n)
     f = rng.standard_normal((n, 6)) * np.array([5, 5, 5, 1, 1, 1.0])
-    _, ref = _gram_reference(g, traj, f)
     q, qd, qdd = soa(traj, torch.float32)
     fd = torch.as_tensor(f, dtype=torch.float32, device="cuda").t().contiguous()
-    for no_tma in (False, True):
-        m = model_from_golden(g, no_tma=no_tma)
-        pack = m.regressor_gram(q, qd, qdd, fd).cpu().numpy()
-        assert np.abs(pack[:100] - ref[:100]).max() < 1e-4 * np.abs(ref[:100]).max()
-        assert np.abs(pack[100:110] - ref[100:110]).max() < 1e-4 * np.abs(ref[:100]).max()
-        assert pack[111] == n
+    for fname, path in (("ref_inverse_hammer.npz", "seq_iso"), ("ref_inverse_generic_nj6.npz", "generic")):
+        g = load_golden(fname)
+        _, ref = _gram_reference(g, traj, f)
+        for no_tma in (False, True):
+            m = model_from_golden(g, no_tma=no_tma)
+            assert m.kernel_path == path
+            pack = m.regressor_gram(q, qd, qdd, fd).cpu().numpy()
+            assert np.abs(pack[:100] - ref[:100]).max() < 1e-4 * np.abs(ref[:100]).max()
+            assert np.abs(pack[100:110] - ref[100:110]).max() < 1e-4 * np.abs(ref[:100]).max()
+            assert pack[111] == n
 
 
 def _gram_reference(g, traj, f):

@@ -195,18 +195,13 @@ def test_fast_and_generic_kernels_agree_at_scale():
 
 def test_rigid_variant_of_the_fast_path():
     """Same kinematic structure with non-isotropic link inertias selects the SEQ_RIGID kernel; checked against the C oracle."""
+    from model_classes import rigid_link_simats
     from oracle import build_c
     from rigid_body_manipulation_b200.engine import Model
 
     g = load_golden("ref_inverse_hammer.npz")
-    sim = g["simats"].copy()
     rng = np.random.default_rng(5)
-    for k in range(1, 6):  # give links 1-5 an offset centre of mass and a full inertia tensor (still a physical rigid body)
-        m, c = 8.0 + k, rng.uniform(-0.1, 0.1, 3)
-        A = rng.standard_normal((3, 3)) * 0.1
-        Ic = A @ A.T + 0.05 * np.eye(3)
-        cx = np.array([[0, -c[2], c[1]], [c[2], 0, -c[0]], [-c[1], c[0], 0]])
-        sim[k] = np.block([[m * np.eye(3), -m * cx], [m * cx, Ic + m * (c @ c * np.eye(3) - np.outer(c, c))]])
+    sim = rigid_link_simats(g["simats"], rng)  # links 1-5: offset centre of mass and a full inertia tensor (still physical rigid bodies)
     mdl = Model(g["hposes_Rt"], sim, g["uscrews"], g["twist_0"], g["dtwist_0"])
     assert mdl.kernel_path == "seq_rigid"
     traj = sample_states(rng, 5000)
@@ -295,6 +290,9 @@ def test_fp32_soa_sizes_and_flags(n, no_tma):
     assert rel_err(tau.t().cpu().numpy(), ref).max() < TOL32
     tau_tw, V, dV = m.rnea(q, qd, qdd, want_twists=True)
     assert torch.equal(tau, tau_tw)
+    tw = rv.inverse_batched(traj, g["hposes_Rt"], g["simats"], g["uscrews"], g["twist_0"], g["dtwist_0"])
+    assert rel_err(V.t().cpu().numpy(), tw["twists"][:, 6]).max() < TOL32
+    assert rel_err(dV.t().cpu().numpy(), tw["dtwists"][:, 6]).max() < TOL32
     tau_aos = m.rnea_aos(torch.as_tensor(traj, dtype=torch.float32, device="cuda"))
     assert rel_err(tau_aos.cpu().numpy(), ref).max() < TOL32
     tau_aos64 = m.rnea_aos(torch.as_tensor(traj, device="cuda"))

@@ -5,6 +5,7 @@ Launch / memory / TMA behaviour is covered by the -m gpu suite through the real 
 import numpy as np
 import pytest
 
+import model_classes
 from conftest import load_golden
 from rigid_body_manipulation_b200 import engine
 
@@ -62,15 +63,31 @@ def test_model_analysis_fallbacks():
         engine.analyze_model(g["hposes_Rt"][:-1], g["simats"], g["uscrews"], g["twist_0"], g["dtwist_0"])
 
 
-@pytest.mark.parametrize("t", TARGETS)
+def _classes_reference(name):
+    """A tests/model_classes.py class in the form of a golden: sampled states and the vectorised oracle's answers."""
+    from oracle import rnea_vec as rv
+
+    mc = model_classes.build(name)
+    rng = np.random.default_rng(13)
+    n = 500
+    traj = model_classes.sample_states(rng, n)
+    out = rv.inverse_batched(traj, mc.hposes_Rt, mc.simats, mc.uscrews, mc.twist_0, mc.dtwist_0)
+    return dict(traj=traj, tau=out["tau"], twists=out["twists"], dtwists=out["dtwists"]), model_classes.analyze(mc)
+
+
+@pytest.mark.parametrize("t", TARGETS + list(model_classes.CLASSES))
 def test_fast_recursion_matches_reference_golden(t):
-    g = load_golden(f"ref_inverse_{t}.npz")
-    path, fast, _ = analyze(g)
+    if t in model_classes.CLASSES:
+        g, (path, fast, _) = _classes_reference(t)
+    else:
+        g = load_golden(f"ref_inverse_{t}.npz")
+        path, fast, _ = analyze(g)
     tau, V, dV = host_harness.fast_rnea(path, fast, g["traj"])
     assert rel_err(tau, g["tau"]).max() < 1e-12
     assert rel_err(V, g["twists"][:, 6]).max() < 1e-12 and rel_err(dV, g["dtwists"][:, 6]).max() < 1e-12
-    tau32, _, _ = host_harness.fast_rnea(path, fast, g["traj"], dtype=np.float32)
+    tau32, V32, dV32 = host_harness.fast_rnea(path, fast, g["traj"], dtype=np.float32)
     assert rel_err(tau32, g["tau"]).max() < 1e-4
+    assert rel_err(V32, g["twists"][:, 6]).max() < 1e-4 and rel_err(dV32, g["dtwists"][:, 6]).max() < 1e-4
     # the all-rigid descriptor evaluates the same model
     tau_r, _, _ = host_harness.fast_rnea("seq_rigid", fast, g["traj"])
     assert rel_err(tau_r, g["tau"]).max() < 1e-12
