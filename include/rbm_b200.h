@@ -48,10 +48,7 @@ enum { RBM_MAX_JOINTS_ABI = 16 };
 /* rbm_model_create flags */
 enum {
   RBM_FLAG_FORCE_GENERIC = 1, /* never select a structure-specialised kernel */
-  RBM_FLAG_NO_TMA = 2,        /* never use the bulk-async (TMA) pipelined kernel variants */
-  RBM_FLAG_GRAM_TENSOR_CORES = 4 /* fp32-mode Gram on the tensor cores (tcgen05.mma kind::tf32 with an exact hi/lo operand split,
-                                    accumulator in TMEM; csrc/rbm_gram_tc.cu).  Parity-correct but measured slower than the default
-                                    register kernel on B200 (34.5 vs 47.3 G samples/s), hence opt-in. */
+  RBM_FLAG_NO_TMA = 2         /* never use the bulk-async (TMA) pipelined kernel variants */
 };
 
 /* kernel path chosen for a model (rbm_model_kernel_path) */

@@ -18,7 +18,6 @@ HEADER = os.path.join(os.path.dirname(_PKG), "include", "rbm_b200.h")
 RBM_OK, RBM_ERR_INVALID, RBM_ERR_CUDA, RBM_ERR_UNSUPPORTED, RBM_ERR_NCCL = 0, -1, -2, -3, -4
 FLAG_FORCE_GENERIC = 1
 FLAG_NO_TMA = 2
-FLAG_GRAM_TENSOR_CORES = 4
 PATH_NAMES = {0: "generic", 1: "seq_iso", 2: "seq_rigid"}
 
 

@@ -19,7 +19,7 @@ ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 OBJ = os.path.join(PKG, "_build")
 LIB = os.path.join(PKG, "librbm_b200.so")
-SOURCES = ["rbm_abi.cu", "rbm_rnea.cu", "rbm_regressor.cu", "rbm_gram_tc.cu", "rbm_linearize.cu", "rbm_setup.cu", "rbm_nccl.cu"]
+SOURCES = ["rbm_abi.cu", "rbm_rnea.cu", "rbm_regressor.cu", "rbm_linearize.cu", "rbm_setup.cu", "rbm_nccl.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -345,7 +345,6 @@ int analyze_model(const char* who, int nj, const double* hposes_Rt, const double
     if (!std::isfinite(uscrews[i])) return invalid(w + ": non-finite screw");
   m->nj = nj;
   m->no_tma = (flags & RBM_FLAG_NO_TMA) != 0;
-  m->gram_tc = (flags & RBM_FLAG_GRAM_TENSOR_CORES) != 0;
   m->gp64.assign(np, 0.0);
   double* g = m->gp64.data();
   static const double ident[12] = {1, 0, 0, 0, 1, 0, 0, 0, 1, 0, 0, 0};

@@ -15,7 +15,6 @@ struct rbm_model {
   int path = rbm::PATH_GENERIC;
   int device = 0;
   bool no_tma = false;  // RBM_FLAG_NO_TMA: keep to the direct-load kernels (A/B comparisons, debugging)
-  bool gram_tc = false; // RBM_FLAG_GRAM_TENSOR_CORES: fp32-mode Gram through tcgen05 (rbm_gram_tc.cu)
   std::vector<double> gp64;  // generic packed parameters (rbm_model.cuh layout), host copies
   std::vector<float> gp32;
   double* d_gp64 = nullptr;  // device copies, staged into shared memory by every block
@@ -109,11 +108,6 @@ int launch_regressor_gram(const rbm_model* m, const T* q, const T* qd, const T* 
 template <class T>
 int launch_regressor_gram_grouped(const rbm_model* m, const T* q, const T* qd, const T* qdd, const T* f, int64_t frame_stride, int64_t f_frame_stride,
                                   int64_t n_frames, double* packs, int64_t n_groups, int64_t ld, int64_t ld_out, cudaStream_t st);
-
-// tensor-core Gram, fp32 mode (rbm_gram_tc.cu): per-CTA partials in the 70-entry layout of rbm_gram.cuh, `grid` from tc_gram_grid
-int tc_gram_grid(int sms, int64_t n);
-int launch_regressor_gram_tc(const rbm_model* m, const float* q, const float* qd, const float* qdd, const float* f, double* partials, int64_t n, int64_t ld,
-                             int grid, cudaStream_t st);
 
 // launcher (rbm_linearize.cu)
 template <class T>

@@ -241,7 +241,7 @@ __global__ void __launch_bounds__(kGramBlock, 1) k_regressor_gram(const __grid_c
 //                                                                     28.2 / 44.2   (ptxas front-loads the FMAs; +14 % instructions)
 //            warp-pair split of the 70 accumulators (12 warps / SM, 162 registers, 17 % more FP64 work)   29.9 / 43.2
 //            dedicated TMA producer warpgroup, consumers without a CTA barrier                              30.1 /  --
-//            fp32 on the tensor cores (tcgen05 tf32 hi/lo, rbm_gram_tc.cu)                                   -- / 34.5
+//            fp32 on the tensor cores (tcgen05 tf32 hi/lo, experiments/k_regressor_gram_tc.cu.inc)           -- / 34.5
 //            512-sample tiles, two samples per thread, 2 stages (THIS KERNEL)                              33.6 / 54.9
 // ncu of the 256-sample kernel (profiles/r2_gram_v2_ncu_full.csv, r2_gram32_v2_ncu_full.csv): fp64 FP64 pipe 60 % active, issue slots 49 %,
 // 19 % of the loop's stall samples in the per-tile hand-over; fp32 issue slots 75 % busy -- which is what the larger tile attacks.
@@ -541,16 +541,6 @@ int launch_regressor_gram(const rbm_model* m, const T* q, const T* qd, const T* 
                         !m->no_tma;
     const int dev = (m->device >= 0 && m->device < 64) ? m->device : 0;
     const bool diag = P.sen_diag != T(0);
-    if constexpr (sizeof(T) == 4) {
-      if (tma_ok && m->gram_tc) {  // fp32 mode on the tensor cores (rbm_gram_tc.cu), opt-in: measured slower than the register kernel
-        grid = tc_gram_grid(sm_count(m->device), n);
-        int rc = launch_regressor_gram_tc(m, q, qd, qdd, f, partials, n, ld, grid, st);
-        if (rc != RBM_OK) return rc;
-        k_gram_finalize<<<1, 128, 0, st>>>(partials, grid, (double)n, pack);
-        RBM_CUDA_TRY(cudaGetLastError());
-        return RBM_OK;
-      }
-    }
     if (tma_ok) {
       const int64_t tiles = n / kTmaTile;  // the ragged tail rides with the CTA that would have received the next tile
       const int64_t cap = (int64_t)sm_count(m->device) * (sizeof(T) == 4 ? 2 : 1);  // fp64 254 registers: 1 CTA / SM; fp32 128: 2

@@ -5,7 +5,6 @@
 // re-read.  Rows the result does not depend on are not loaded (SoaRows): a tau-only launch on the
 // sequential structure moves 18 * sizeof(T) bytes per sample of the 24 the rows hold.
 #include <atomic>
-#include <cstdlib>
 #include <cstring>
 
 #include "rbm_async.cuh"
@@ -20,14 +19,6 @@ constexpr int kBlock = 128;
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait_prior_grids() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
-static bool pdl_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("RBM_NO_PDL");
-    return !(e && e[0] == '1');
-  }();
-  return on;
-}
-
 // launch with programmatic stream serialisation allowed: the grid may start (and park in griddepcontrol.wait) while the
 // previous kernel of the stream is still draining, which removes the launch gap between back-to-back batches
 template <class... KArgs, class... Args>
@@ -39,7 +30,7 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), unsigned grid, unsigned 
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);

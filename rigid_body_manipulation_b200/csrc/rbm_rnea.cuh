@@ -456,19 +456,12 @@ RBM_HD void regressor_x(const T* V, const T* dV, T (&x)[3]) {
   x[1] = dV[1] + (wz * vx - wx * vz);
   x[2] = dV[2] + (wx * vy - wy * vx);
 }
-// quadratic angular-velocity terms ww = (xx, yy, zz, xy, yz, zx)
 template <class T>
-RBM_HD void regressor_products(const T* w, T (&ww)[6]) {
+RBM_HD void regressor_blocks_xwl(const T (&x)[3], const T* w, const T* l, T (&top)[3][4], T (&bot)[3][9]) {
   const T wx = w[0], wy = w[1], wz = w[2];
-  ww[0] = wx * wx; ww[1] = wy * wy; ww[2] = wz * wz; ww[3] = wx * wy; ww[4] = wy * wz; ww[5] = wz * wx;
-}
-// the blocks are LINEAR in the features (x, dw, ww) with coefficients 0 / +-1 (the tensor-core Gram kernel relies on this: the Gram of
-// [Y f] is a fixed linear image of the second moments of the 18 features (x, dw, ww, f), rbm_gram_tc.cu)
-template <class T>
-RBM_HD void regressor_blocks_feat(const T (&x)[3], const T* l, const T (&ww)[6], T (&top)[3][4], T (&bot)[3][9]) {
+  const T xx = wx * wx, yy = wy * wy, zz = wz * wz, xy = wx * wy, yz = wy * wz, zx = wz * wx;
   const T lx = l[0], ly = l[1], lz = l[2];
   const T x0 = x[0], x1 = x[1], x2 = x[2];
-  const T xx = ww[0], yy = ww[1], zz = ww[2], xy = ww[3], yz = ww[4], zx = ww[5];
   top[0][0] = x0; top[0][1] = -(yy + zz); top[0][2] = xy - lz;     top[0][3] = zx + ly;
   top[1][0] = x1; top[1][1] = xy + lz;    top[1][2] = -(xx + zz);  top[1][3] = yz - lx;
   top[2][0] = x2; top[2][1] = zx - ly;    top[2][2] = yz + lx;     top[2][3] = -(xx + yy);
@@ -480,12 +473,6 @@ RBM_HD void regressor_blocks_feat(const T (&x)[3], const T* l, const T (&ww)[6],
   bot[0][3] = lx;   bot[0][4] = -yz;  bot[0][5] = yz;   bot[0][6] = ly - zx; bot[0][7] = yy - zz; bot[0][8] = lz + xy;
   bot[1][3] = zx;   bot[1][4] = ly;   bot[1][5] = -zx;  bot[1][6] = lx + yz; bot[1][7] = lz - xy; bot[1][8] = zz - xx;
   bot[2][3] = -xy;  bot[2][4] = xy;   bot[2][5] = lz;   bot[2][6] = xx - yy; bot[2][7] = ly + zx; bot[2][8] = lx - yz;
-}
-template <class T>
-RBM_HD void regressor_blocks_xwl(const T (&x)[3], const T* w, const T* l, T (&top)[3][4], T (&bot)[3][9]) {
-  T ww[6];
-  regressor_products(w, ww);
-  regressor_blocks_feat(x, l, ww, top, bot);
 }
 template <class T>
 RBM_HD void regressor_blocks(const T* V, const T* dV, T (&top)[3][4], T (&bot)[3][9]) {

@@ -80,7 +80,7 @@ class Model:
     """Device-resident model constants (opaque `rbm_model*`) for one CUDA device."""
 
     def __init__(self, hposes_body_parent, simats_body, uscrews_body, twist_0, dtwist_0, wrench_tip=None,
-                 pose_tip_ee=None, pose_sen_llj=None, device=None, force_generic=False, no_tma=False, gram_tensor_cores=False):
+                 pose_tip_ee=None, pose_sen_llj=None, device=None, force_generic=False, no_tma=False):
         lib = _lib.load()
         self.uscrews = _f64(uscrews_body)
         if self.uscrews.ndim != 2 or self.uscrews.shape[1] != 6:
@@ -101,8 +101,8 @@ class Model:
         handle = C.c_void_p()
         rc = lib.rbm_model_create(nj, _ptr(self.hposes_Rt), _ptr(self.simats), _ptr(self.uscrews), _ptr(self.twist_0),
                                   _ptr(self.dtwist_0), _ptr(self.wrench_tip), _ptr(self.pose_tip), _ptr(self.pose_sen),
-                                  (_lib.FLAG_FORCE_GENERIC if force_generic else 0) | (_lib.FLAG_NO_TMA if no_tma else 0)
-                                  | (_lib.FLAG_GRAM_TENSOR_CORES if gram_tensor_cores else 0), self.device.index, C.byref(handle))
+                                  (_lib.FLAG_FORCE_GENERIC if force_generic else 0) | (_lib.FLAG_NO_TMA if no_tma else 0),
+                                  self.device.index, C.byref(handle))
         _lib.check(rc, "rbm_model_create")
         self._h = handle
         self._lib = lib

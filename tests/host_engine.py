@@ -24,7 +24,7 @@ class Model:
     """Same constructor and the methods the drop-in packages call (rnea_full_host, linearize), evaluated on the host."""
 
     def __init__(self, hposes_body_parent, simats_body, uscrews_body, twist_0, dtwist_0, wrench_tip=None, pose_tip_ee=None, pose_sen_llj=None,
-                 device=None, force_generic=False, no_tma=False, gram_tensor_cores=False):
+                 device=None, force_generic=False, no_tma=False):
         self.uscrews = np.ascontiguousarray(uscrews_body, dtype=np.float64)
         self.nj = self.uscrews.shape[0]
         self.analysis = real_engine.analyze_model(hposes_body_parent, simats_body, uscrews_body, twist_0, dtwist_0, wrench_tip, pose_tip_ee, pose_sen_llj,

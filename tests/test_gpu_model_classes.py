@@ -2,8 +2,7 @@
 
 The packaged robot selects SEQ_ISO with a sign-pattern sensor adjoint (SEN_DIAG) and gravity along z; these classes select the SEQ_RIGID
 instantiations, the SEN_DIAG = false ones and a tilted base acceleration.  Sizes are chosen per entry point to reach each dispatch
-branch (paired / unpaired / one-sample fp32 SoA, plain / TMA AoS, direct / TMA / tensor-core Gram with whole tiles and both half-tile
-tails).  The packaged hammer model runs between the classes' calls of the AoS and Gram launchers; the Gram launcher raises the shared
+branch (paired / unpaired / one-sample fp32 SoA, plain / TMA AoS, direct / TMA Gram with whole tiles and both half-tile tails).  The packaged hammer model runs between the classes' calls of the AoS and Gram launchers; the Gram launcher raises the shared
 memory limit of each kernel variant in its own cached slot, so this also switches between those slots.  Tolerances are the suite's
 bars: 1e-9 in fp64, 1e-4 in fp32, norm-wise per sample (gpu_util.rel_err)."""
 import ctypes as C
@@ -26,7 +25,7 @@ pytestmark = pytest.mark.gpu
 TOL64 = 1e-9
 TOL32 = 1e-4
 N_GRAM = 300_004        # 585 whole 512-sample TMA tiles + a 484-sample tail that reaches both half-tiles; a multiple of 4, so that the
-                        # fp32 row pitch (n * 4 bytes) is 16-byte aligned too and fp32 takes the TMA and tensor-core kernels as well
+                        # fp32 row pitch (n * 4 bytes) is 16-byte aligned too and fp32 takes the TMA kernel as well
 N_RNEA = 4096 + 77      # 32 AoS tiles of 128 + a ragged 77; odd, so fp32 SoA with ld = n takes the one-sample kernel
 INPUT_GAIN = [10.0, 10.0, 10.0, 1e4, 1e4, 1e4]             # configurations/base.yaml controller.input_gain
 DISP = [0.2, 1.4, 0.6, np.pi, 0.0, 18.8495559215]          # configurations/base.yaml planner.displacements
@@ -207,14 +206,13 @@ def test_regressor_from_traj(case, dtype, tol):
     assert rel_err(host(out["wrench"]), case.Y[:n] @ case.mc.phi).max() < tol
 
 
-GRAM_MODES = {"fp64": (torch.float64, {}, TOL64), "fp32": (torch.float32, {}, TOL32),
-              "fp32_tc": (torch.float32, dict(gram_tensor_cores=True), TOL32)}
+GRAM_MODES = {"fp64": (torch.float64, {}, TOL64), "fp32": (torch.float32, {}, TOL32)}
 
 
 @pytest.mark.parametrize("mode", list(GRAM_MODES))
 @pytest.mark.parametrize("n,no_tma", [(511, False), (4096, False), (4097, False), (N_GRAM, False), (N_GRAM, True)])
 def test_regressor_gram(case, mode, n, no_tma):
-    """511 and odd 4097 take the direct-load kernel; 4096 whole TMA (or, with gram_tensor_cores, tensor-core) tiles; N_GRAM whole tiles
+    """511 and odd 4097 take the direct-load kernel; 4096 whole TMA tiles; N_GRAM whole tiles
     + a tail over both half-tiles, in fp64 and fp32 alike (16-byte aligned rows); no_tma=True the direct-load kernel at N_GRAM."""
     dtype, flags, tol = GRAM_MODES[mode]
     m = make_model(case.mc, no_tma=no_tma, **flags)

@@ -45,7 +45,7 @@ def test_fused_regressor_from_trajectory(fname, force_generic):
     assert rel_err(o32["wrench"].t().cpu().numpy(), g["regressor"] @ phi).max() < 1e-4
 
 
-@pytest.mark.parametrize("n", [4096, 262_144 + 256 * 5 + 100])
+@pytest.mark.parametrize("n", [100, 256, 4096, 262_144 + 256 * 5 + 100, 2_100_000])
 def test_gram_fp32_mode(n):
     """The fast model (TMA and direct-load fp32 kernels) and a generic six-joint model (k_regressor_gram<float, PATH_GENERIC>)."""
     rng = np.random.default_rng(n)
@@ -229,59 +229,13 @@ def test_per_object_grams_for_all_packaged_targets():
         assert (np.abs(r.phi - phi) / scale).max() < 1e-7, (name, r.phi, phi)
 
 
-@pytest.mark.parametrize("n", [100, 256, 4096, 262_144 + 256 * 5 + 100, 2_100_000])
-def test_gram_fp32_on_the_tensor_cores(n):
-    """RBM_FLAG_GRAM_TENSOR_CORES (csrc/rbm_gram_tc.cu): second moments of the 18 regressor features through tcgen05.mma kind::tf32
-    with an exact hi/lo operand split, accumulator in TMEM, flushed to fp64 every 2048 samples.  Same bar as the register fp32 kernel
-    (1e-4 of the largest entry, north_star's fp32 tolerance); ragged tails, sub-tile batches and multi-tile-per-CTA sizes."""
-    g = load_golden("ref_inverse_hammer.npz")
-    rng = np.random.default_rng(n)
-    traj = sample_states(rng, n)
-    f = rng.standard_normal((n, 6)) * np.array([5, 5, 5, 1, 1, 1.0])
-    _, ref = _gram_reference(g, traj, f)
-    q, qd, qdd = soa(traj, torch.float32)
-    fd = torch.as_tensor(f, dtype=torch.float32, device="cuda").t().contiguous()
-    m = model_from_golden(g, gram_tensor_cores=True)
-    pack = m.regressor_gram(q, qd, qdd, fd).cpu().numpy()
-    scale = np.abs(ref[:100]).max()
-    assert np.abs(pack[:100] - ref[:100]).max() < 1e-4 * scale
-    assert np.abs(pack[100:110] - ref[100:110]).max() < 1e-4 * scale
-    assert abs(pack[110] - ref[110]) < 1e-4 * ref[110]
-    assert pack[111] == n
-    G = pack[:100].reshape(10, 10)
-    assert np.array_equal(G, G.T)
-    assert np.array_equal(pack, m.regressor_gram(q, qd, qdd, fd).cpu().numpy())  # fixed reduction order here too
-    # the register fp32 kernel on the same data: the two fp32 modes agree to well inside the bar
-    reg = model_from_golden(g).regressor_gram(q, qd, qdd, fd).cpu().numpy()
-    assert np.abs(pack[:111] - reg[:111]).max() < 5e-5 * scale
-
-
-def test_tensor_core_gram_identifies_like_the_register_kernel():
-    """TF32 characterisation on phi-hat (VERDICT r1 item 4c): exact-recovery data, 2^21 samples; the estimate from the tensor-core
-    Gram against the one from the register fp32 Gram and against the truth."""
-    g = load_golden("ref_inverse_uniform_gearbox.npz")
-    n = 1 << 21
-    traj = sample_states(np.random.default_rng(42), n)
-    q, qd, qdd = soa(traj, torch.float32)
-    phi_true = np.array([0.585, -0.0032, 1.9e-5, -8e-6, 3.85e-3, 2.9e-3, 3.0e-3, 1e-5, 2e-5, -1e-5])
-    scale = np.array([1, 1e-2, 1e-2, 1e-2, 1e-3, 1e-3, 1e-3, 1e-3, 1e-3, 1e-3])
-    est = {}
-    for name, kw in (("tc", dict(gram_tensor_cores=True)), ("reg", {})):
-        m = model_from_golden(g, **kw)
-        f = m.regressor_from_traj(q, qd, qdd, want_rows=False, phi=phi_true)["wrench"]
-        est[name] = identification.solve(m.regressor_gram(q, qd, qdd, f))
-        assert est[name].rank == 10
-        assert (np.abs(est[name].phi - phi_true) / scale).max() < 2e-3
-    assert (np.abs(est["tc"].phi - est["reg"].phi) / scale).max() < 2e-3
-
-
-@pytest.mark.parametrize("dtype,tc,tol", [(torch.float64, False, 1e-12), (torch.float32, False, 2e-6), (torch.float32, True, 5e-5)])
-def test_gram_is_additive_at_the_configs2_size(dtype, tc, tol):
+@pytest.mark.parametrize("dtype,tol", [(torch.float64, 1e-12), (torch.float32, 2e-6)])
+def test_gram_is_additive_at_the_configs2_size(dtype, tol):
     """BASELINE configs[2] per-GPU share (12.5 M samples), size-independent properties: the pack of the whole batch equals the sum of the
     packs of its two halves (what the multi-GPU all-reduce relies on), the sample count is exact, and a batch that is the same 4096
     samples repeated gives 3052 x the pack of one copy (+ the ragged remainder), so every tile of the persistent grid is accounted for."""
     g = load_golden("ref_inverse_uniform_gearbox.npz")
-    m = model_from_golden(g, gram_tensor_cores=tc)
+    m = model_from_golden(g)
     n = 12_500_000
     gen = torch.Generator(device="cuda").manual_seed(7)
     q = (torch.rand((6, n), generator=gen, device="cuda", dtype=dtype) * 2 - 1) * 6
