@@ -197,6 +197,30 @@ RBM_API int rbm_regressor_gram_f64(const rbm_model* m, const double* q, const do
 RBM_API int rbm_regressor_gram_f32(const rbm_model* m, const float* q, const float* qd, const float* qdd, const float* f, double* gram_pack,
                            void* workspace, size_t workspace_bytes, int64_t n, int64_t ld, void* stream);
 
+/* ---- payload identification from joint torques ------------------------------------------------------
+ * The same 10 parameters phi, in the sensor frame of the model's pose_sen_Rt, identified from joint torques instead of the F/T
+ * sensor.  `m` is the robot WITHOUT the payload; the payload hangs off the last link.  RNEA is linear in the link inertias, so
+ *   tau(q, qd, qdd) = tau0(q, qd, qdd) + Phi(q, qd, qdd) phi,   Phi = J_s^T Y_s  (nj x 10)
+ * with tau0 the model's own inverse dynamics, Y_s the sensor-frame regressor of rbm_regressor_from_traj_* and J_s the last link's
+ * Jacobian in the sensor frame.
+ *   q, qd, qdd : [nj][ld]     Phi : [n][nj][10] (row-major per sample) or NULL     tau0 : [nj][ld] or NULL
+ * On a fast-path model neither q[0..2] nor qd[0..2] is read (Phi and tau0 do not depend on them; the caller may leave those rows
+ * unset), rows 0..2 of Phi are zero in columns 4..9, and tau0 is bit-identical to rbm_rnea_*'s tau. */
+RBM_API int rbm_payload_regressor_f64(const rbm_model* m, const double* q, const double* qd, const double* qdd, double* Phi, double* tau0, int64_t n,
+                              int64_t ld, void* stream);
+RBM_API int rbm_payload_regressor_f32(const rbm_model* m, const float* q, const float* qd, const float* qdd, float* Phi, float* tau0, int64_t n,
+                              int64_t ld, void* stream);
+/* Normal equations of min ||Phi phi - (tau - tau0)||^2 over the batch, in the pack layout of rbm_regressor_gram_*:
+ *   gram_pack [112] (device, double) = [Phi^T Phi (100, row-major) | Phi^T r (10) | r^T r | n],  r = tau - tau0
+ *   tau [nj][ld]: measured joint torques.  workspace: rbm_gram_workspace_bytes(m, n) bytes, as for rbm_regressor_gram_*.
+ * The pack solves, sums and all-reduces like an F/T pack (rbm_allreduce_gram*); packs of the two routes may be added.  Fixed
+ * reduction order, no atomics: bit-reproducible for a given n.  The fast path reads 18 rows per sample (q[3..5], qd[3..5], qdd, tau).
+ * fp32 forms the rows in float and accumulates in double every 64 samples.  n = 0 yields a zero pack. */
+RBM_API int rbm_payload_gram_f64(const rbm_model* m, const double* q, const double* qd, const double* qdd, const double* tau, double* gram_pack,
+                         void* workspace, size_t workspace_bytes, int64_t n, int64_t ld, void* stream);
+RBM_API int rbm_payload_gram_f32(const rbm_model* m, const float* q, const float* qd, const float* qdd, const float* tau, double* gram_pack,
+                         void* workspace, size_t workspace_bytes, int64_t n, int64_t ld, void* stream);
+
 /* One Gram pack per GROUP (environment / object) for logs stored frame-major: sample `fr` of group g has its row k at
  *   x[fr * frame_stride + k * ld + g]  (x = q, qd, qdd: nj rows)   and   f[fr * f_frame_stride + k * ld + g]  (6 rows)
  * e.g. the frame log of rbm_closed_loop_f64 (q = frames, qd = frames + nj ld, qdd = frames + 2 nj ld, f = frames + (3 nj + 12) ld,

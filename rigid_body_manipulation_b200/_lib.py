@@ -75,6 +75,10 @@ SIGNATURES = {
     "rbm_gram_workspace_bytes": (C.c_size_t, [_vp, _i64]),
     "rbm_regressor_gram_f64": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_size_t, _i64, _i64, _vp]),
     "rbm_regressor_gram_f32": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_size_t, _i64, _i64, _vp]),
+    "rbm_payload_regressor_f64": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
+    "rbm_payload_regressor_f32": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp]),
+    "rbm_payload_gram_f64": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_size_t, _i64, _i64, _vp]),
+    "rbm_payload_gram_f32": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_size_t, _i64, _i64, _vp]),
     "rbm_nccl_available": (C.c_int, []),
     "rbm_nccl_unique_id": (C.c_int, [_vp]),
     "rbm_nccl_comm_create": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.POINTER(_vp)]),

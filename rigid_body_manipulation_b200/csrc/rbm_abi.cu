@@ -673,6 +673,30 @@ int regressor_gram(const char* name, const rbm_model* m, const T* q, const T* qd
   RBM_CUDA_TRY(guard.status());
   return launch_regressor_gram<T>(m, q, qd, qdd, f, pack, static_cast<double*>(ws), n, ld, (cudaStream_t)stream);
 }
+template <class T>
+int payload_regressor(const char* name, const rbm_model* m, const T* q, const T* qd, const T* qdd, T* Phi, T* tau0, int64_t n, int64_t ld, void* stream) {
+  if (!m) return invalid(std::string(name) + ": model is NULL");
+  if (n < 0) return invalid(std::string(name) + ": n < 0");
+  if (n == 0) return RBM_OK;
+  if (!q || !qd || !qdd) return invalid(std::string(name) + ": NULL batch pointer");
+  if (ld < n) return invalid(std::string(name) + ": ld < n");
+  DeviceGuard guard(m->device);
+  RBM_CUDA_TRY(guard.status());
+  return launch_payload_regressor<T>(m, q, qd, qdd, Phi, tau0, n, ld, (cudaStream_t)stream);
+}
+template <class T>
+int payload_gram(const char* name, const rbm_model* m, const T* q, const T* qd, const T* qdd, const T* tau, double* pack, void* ws, size_t ws_bytes,
+                 int64_t n, int64_t ld, void* stream) {
+  if (!m) return invalid(std::string(name) + ": model is NULL");
+  if (n < 0) return invalid(std::string(name) + ": n < 0");
+  if (!pack || !ws) return invalid(std::string(name) + ": NULL gram_pack / workspace");
+  if (n > 0 && (!q || !qd || !qdd || !tau)) return invalid(std::string(name) + ": NULL batch pointer");
+  if (ld < n) return invalid(std::string(name) + ": ld < n");
+  if (ws_bytes < rbm_gram_workspace_bytes(m, n)) return invalid(std::string(name) + ": workspace too small (see rbm_gram_workspace_bytes)");
+  DeviceGuard guard(m->device);
+  RBM_CUDA_TRY(guard.status());
+  return launch_payload_gram<T>(m, q, qd, qdd, tau, pack, static_cast<double*>(ws), n, ld, (cudaStream_t)stream);
+}
 }  // namespace
 
 extern "C" {
@@ -697,6 +721,23 @@ int rbm_regressor_gram_f64(const rbm_model* m, const double* q, const double* qd
 int rbm_regressor_gram_f32(const rbm_model* m, const float* q, const float* qd, const float* qdd, const float* f, double* gram_pack, void* workspace,
                            size_t workspace_bytes, int64_t n, int64_t ld, void* stream) {
   return regressor_gram<float>("rbm_regressor_gram_f32", m, q, qd, qdd, f, gram_pack, workspace, workspace_bytes, n, ld, stream);
+}
+
+int rbm_payload_regressor_f64(const rbm_model* m, const double* q, const double* qd, const double* qdd, double* Phi, double* tau0, int64_t n, int64_t ld,
+                              void* stream) {
+  return payload_regressor<double>("rbm_payload_regressor_f64", m, q, qd, qdd, Phi, tau0, n, ld, stream);
+}
+int rbm_payload_regressor_f32(const rbm_model* m, const float* q, const float* qd, const float* qdd, float* Phi, float* tau0, int64_t n, int64_t ld,
+                              void* stream) {
+  return payload_regressor<float>("rbm_payload_regressor_f32", m, q, qd, qdd, Phi, tau0, n, ld, stream);
+}
+int rbm_payload_gram_f64(const rbm_model* m, const double* q, const double* qd, const double* qdd, const double* tau, double* gram_pack, void* workspace,
+                         size_t workspace_bytes, int64_t n, int64_t ld, void* stream) {
+  return payload_gram<double>("rbm_payload_gram_f64", m, q, qd, qdd, tau, gram_pack, workspace, workspace_bytes, n, ld, stream);
+}
+int rbm_payload_gram_f32(const rbm_model* m, const float* q, const float* qd, const float* qdd, const float* tau, double* gram_pack, void* workspace,
+                         size_t workspace_bytes, int64_t n, int64_t ld, void* stream) {
+  return payload_gram<float>("rbm_payload_gram_f32", m, q, qd, qdd, tau, gram_pack, workspace, workspace_bytes, n, ld, stream);
 }
 
 int rbm_regressor_gram_grouped_f64(const rbm_model* m, const double* q, const double* qd, const double* qdd, const double* f, int64_t frame_stride,

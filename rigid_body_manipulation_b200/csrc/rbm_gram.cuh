@@ -59,4 +59,31 @@ RBM_HD double gram_pack_entry(const TA* tot, int t) {
   return v;
 }
 
+// ---- joint-torque payload route (rbm_payload.cuh): [Phi r]^T [Phi r], Phi (nj x 10) and r = tau - tau0 per sample ----------------
+constexpr int kPayAcc = 66;  // upper triangle of the 11 x 11 product, row-major i <= j
+
+__host__ __device__ constexpr int tri11(int i, int j) { return i <= j ? i * 11 - i * (i - 1) / 2 + (j - i) : j * 11 - j * (j - 1) / 2 + (i - j); }
+
+// One row [Phi_j | r_j].  A prismatic joint's row is zero in columns 4..9 and touches only the 15 entries among columns {0..3, r}.
+template <class TA, class T>
+RBM_HD void payload_accumulate_row(TA (&acc)[kPayAcc], const T (&phi)[10], T r, bool prismatic) {
+  TA u[11];
+#pragma unroll
+  for (int c = 0; c < 10; ++c) u[c] = (TA)phi[c];
+  u[10] = (TA)r;
+#pragma unroll
+  for (int i = 0; i < 11; ++i)
+#pragma unroll
+    for (int j = i; j < 11; ++j)
+      if (!prismatic || ((i < 4 || i == 10) && (j < 4 || j == 10))) acc[tri11(i, j)] += u[i] * u[j];
+}
+
+// Entry t (0..110) of the pack [Phi^T Phi (100, row-major) | Phi^T r (10) | r^T r] from the 66 accumulators
+template <class TA>
+RBM_HD double payload_pack_entry(const TA* tot, int t) {
+  if (t < 100) return (double)tot[tri11(t / 10, t % 10)];
+  if (t < 110) return (double)tot[tri11(t - 100, 10)];
+  return (double)tot[tri11(10, 10)];
+}
+
 }  // namespace rbm

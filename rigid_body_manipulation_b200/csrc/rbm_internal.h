@@ -106,6 +106,11 @@ template <class T>
 int launch_regressor_gram(const rbm_model* m, const T* q, const T* qd, const T* qdd, const T* f, double* pack, double* partials, int64_t n, int64_t ld,
                           cudaStream_t st);
 template <class T>
+int launch_payload_regressor(const rbm_model* m, const T* q, const T* qd, const T* qdd, T* Phi, T* tau0, int64_t n, int64_t ld, cudaStream_t st);
+template <class T>
+int launch_payload_gram(const rbm_model* m, const T* q, const T* qd, const T* qdd, const T* tau, double* pack, double* partials, int64_t n, int64_t ld,
+                        cudaStream_t st);
+template <class T>
 int launch_regressor_gram_grouped(const rbm_model* m, const T* q, const T* qd, const T* qdd, const T* f, int64_t frame_stride, int64_t f_frame_stride,
                                   int64_t n_frames, double* packs, int64_t n_groups, int64_t ld, int64_t ld_out, cudaStream_t st);
 

@@ -15,6 +15,7 @@
 #include "rbm_async.cuh"
 #include "rbm_internal.h"
 #include "rbm_gram.cuh"
+#include "rbm_payload.cuh"
 #include "rbm_rnea.cuh"
 
 namespace rbm {
@@ -141,9 +142,10 @@ __global__ void __launch_bounds__(kRowsBlock) k_regressor_from_traj(const __grid
 // bot_nz, gram_accumulate, gram_pack_entry: rbm_gram.cuh (shared with the host harness)
 
 // fp32 only: warp-reduce the float partial sums and add them to the warp's double accumulators in shared memory
-__device__ __forceinline__ void gram_flush_f32(float (&acc)[kAcc], double* red_warp, int lane) {
+template <int N>
+__device__ __forceinline__ void gram_flush_f32(float (&acc)[N], double* red_warp, int lane) {
 #pragma unroll
-  for (int k = 0; k < kAcc; ++k) {
+  for (int k = 0; k < N; ++k) {
     float v = acc[k];
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -153,14 +155,14 @@ __device__ __forceinline__ void gram_flush_f32(float (&acc)[kAcc], double* red_w
 }
 
 // block epilogue: registers -> per-warp doubles in shared memory -> fixed-order sum over warps -> partials[blockIdx]
-template <class T>
-__device__ __forceinline__ void gram_block_epilogue(T (&acc)[kAcc], double (*red)[kAcc], double* __restrict__ partials) {
+template <class T, int N>
+__device__ __forceinline__ void gram_block_epilogue(T (&acc)[N], double (*red)[N], double* __restrict__ partials) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   if constexpr (sizeof(T) == 4) {
     gram_flush_f32(acc, red[warp], lane);
   } else {
 #pragma unroll
-    for (int k = 0; k < kAcc; ++k) {
+    for (int k = 0; k < N; ++k) {
       double v = acc[k];
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -168,11 +170,11 @@ __device__ __forceinline__ void gram_block_epilogue(T (&acc)[kAcc], double (*red
     }
   }
   __syncthreads();
-  if (threadIdx.x < kAcc) {
+  if (threadIdx.x < N) {
     double v = 0.0;
 #pragma unroll
     for (int wq = 0; wq < kGramBlock / 32; ++wq) v += red[wq][threadIdx.x];  // fixed order
-    partials[(int64_t)blockIdx.x * kAcc + threadIdx.x] = v;
+    partials[(int64_t)blockIdx.x * N + threadIdx.x] = v;
   }
 }
 
@@ -400,18 +402,24 @@ __global__ void __launch_bounds__(kGramBlock, sizeof(T) == 4 ? 2 : 1) k_regresso
   gram_block_epilogue<T>(acc, red, partials);
 }
 
-// partials [nblocks][70] -> pack [112] = [Y^T Y (100, row-major) | Y^T f (10) | f^T f | n]
-__global__ void __launch_bounds__(128) k_gram_finalize(const double* __restrict__ partials, int nblocks, double n_samples, double* __restrict__ pack) {
-  __shared__ double tot[kAcc];
-  if (threadIdx.x < kAcc) {
+// partials [nblocks][N] -> fixed-order totals -> pack [112] through `entry` (one thread per pack entry, 128 threads)
+template <int N, class Entry>
+__device__ __forceinline__ void gram_finalize(const double* __restrict__ partials, int nblocks, double n_samples, double* __restrict__ pack, Entry entry) {
+  __shared__ double tot[N];
+  if (threadIdx.x < N) {
     double v = 0.0;
-    for (int b = 0; b < nblocks; ++b) v += partials[(int64_t)b * kAcc + threadIdx.x];  // fixed order
+    for (int b = 0; b < nblocks; ++b) v += partials[(int64_t)b * N + threadIdx.x];  // fixed order
     tot[threadIdx.x] = v;
   }
   __syncthreads();
   const int t = threadIdx.x;
-  if (t < 111) pack[t] = gram_pack_entry(tot, t);
+  if (t < 111) pack[t] = entry(tot, t);
   else if (t == 111) pack[t] = n_samples;
+}
+
+// partials [nblocks][70] -> pack [112] = [Y^T Y (100, row-major) | Y^T f (10) | f^T f | n]
+__global__ void __launch_bounds__(128) k_gram_finalize(const double* __restrict__ partials, int nblocks, double n_samples, double* __restrict__ pack) {
+  gram_finalize<kAcc>(partials, nblocks, n_samples, pack, [](const double* tot, int t) { return gram_pack_entry(tot, t); });
 }
 
 // ---- grouped variant: one Gram pack per GROUP (environment / object), one group per thread ----------------------------------
@@ -450,6 +458,121 @@ __global__ void __launch_bounds__(kRowsBlock) k_regressor_gram_grouped(const __g
 #pragma unroll
   for (int t = 0; t < 111; ++t) out[(int64_t)t * ld_out] = gram_pack_entry(acc, t);
   out[(int64_t)111 * ld_out] = (double)n_frames;
+}
+
+// ---------------------------------------------------------------------------------------------
+// joint-torque payload route (rbm_payload.cuh): tau = tau0 + Phi phi, Phi (nj x 10) per sample
+// ---------------------------------------------------------------------------------------------
+// Fast-path inputs of one sample: q[3..5], qd[3..5], qdd, and (Gram) tau -- q[0..2] and qd[0..2] are never read.
+template <class T>
+__device__ __forceinline__ void payload_load_fast(const T* __restrict__ q, const T* __restrict__ qd, const T* __restrict__ qdd, int64_t s, int64_t ld,
+                                                  T (&rq)[6], T (&rqd)[6], T (&rqdd)[6]) {
+#pragma unroll
+  for (int j = 0; j < 3; ++j) {
+    rq[j] = T(0); rqd[j] = T(0);
+    rq[3 + j] = __ldg(q + (3 + j) * ld + s); rqd[3 + j] = __ldg(qd + (3 + j) * ld + s);
+  }
+#pragma unroll
+  for (int j = 0; j < 6; ++j) rqdd[j] = __ldg(qdd + j * ld + s);
+}
+
+// one sample per thread: Phi [n][nj][10] and / or tau0 [nj][ld] (either may be null)
+template <class T, int PATH>
+__global__ void __launch_bounds__(kRowsBlock) k_payload_regressor(const __grid_constant__ FastParams<T> P, const T* __restrict__ gp, int nj, int nparams,
+                                                                  const T* __restrict__ q, const T* __restrict__ qd, const T* __restrict__ qdd,
+                                                                  T* __restrict__ Phi, T* __restrict__ tau0, int64_t n, int64_t ld) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  T* sp = reinterpret_cast<T*>(smem_raw);
+  if constexpr (PATH == PATH_GENERIC) {
+    for (int i = threadIdx.x; i < nparams; i += blockDim.x) sp[i] = gp[i];
+    __syncthreads();
+  }
+  const int64_t s = (int64_t)blockIdx.x * kRowsBlock + threadIdx.x;
+  if (s >= n) return;
+  if constexpr (PATH == PATH_GENERIC) {
+    T rq[RBM_MAX_JOINTS], rqd[RBM_MAX_JOINTS], rqdd[RBM_MAX_JOINTS], t0[RBM_MAX_JOINTS];
+    for (int j = 0; j < nj; ++j) { rq[j] = __ldg(q + j * ld + s); rqd[j] = __ldg(qd + j * ld + s); rqdd[j] = __ldg(qdd + j * ld + s); }
+    payload_generic<T>(sp, nj, rq, rqd, rqdd, t0, [&](int i, const T (&phi)[10]) {
+      if (Phi) {
+#pragma unroll
+        for (int c = 0; c < 10; ++c) Phi[(s * nj + i) * 10 + c] = phi[c];
+      }
+    });
+    if (tau0)
+      for (int j = 0; j < nj; ++j) tau0[j * ld + s] = t0[j];
+  } else {
+    using D = std::conditional_t<PATH == PATH_SEQ_ISO, SeqIso, SeqRigid>;
+    T rq[6], rqd[6], rqdd[6], t0[6];
+    payload_load_fast(q, qd, qdd, s, ld, rq, rqd, rqdd);
+    auto store = [&](int j, const T (&phi)[10]) {
+      if (Phi) {
+#pragma unroll
+        for (int c = 0; c < 10; ++c) Phi[(s * 6 + j) * 10 + c] = phi[c];
+      }
+    };
+    if (P.sen_diag != T(0)) payload_fast<T, D, true>(P, rq, rqd, rqdd, t0, store);
+    else payload_fast<T, D, false>(P, rq, rqd, rqdd, t0, store);
+    if (tau0) {
+#pragma unroll
+      for (int j = 0; j < 6; ++j) tau0[j * ld + s] = t0[j];
+    }
+  }
+}
+
+// Normal equations of the payload route: the direct-load persistent form of k_regressor_gram with the 66 accumulators of
+// [Phi r]^T [Phi r], r = tau - tau0 (payload_accumulate_row; the fast path's gantry rows add to the 15 entries of columns {0..3, r}).
+template <class T, int PATH, bool SEN_DIAG>
+__global__ void __launch_bounds__(kGramBlock, 1) k_payload_gram(const __grid_constant__ FastParams<T> P, const T* __restrict__ gp, int nj, int nparams,
+                                                                const T* __restrict__ q, const T* __restrict__ qd, const T* __restrict__ qdd,
+                                                                const T* __restrict__ tau, double* __restrict__ partials /* [grid][kPayAcc] */,
+                                                                int64_t n, int64_t ld) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  T* sp = reinterpret_cast<T*>(smem_raw);
+  if constexpr (PATH == PATH_GENERIC) {
+    for (int i = threadIdx.x; i < nparams; i += blockDim.x) sp[i] = gp[i];
+  }
+  __shared__ double red[kGramBlock / 32][kPayAcc];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int k = lane; k < kPayAcc; k += 32) red[warp][k] = 0.0;
+  __syncthreads();
+  T acc[kPayAcc];
+#pragma unroll
+  for (int k = 0; k < kPayAcc; ++k) acc[k] = T(0);
+  const int64_t stride = (int64_t)gridDim.x * kGramBlock;
+  const int64_t first = (int64_t)blockIdx.x * kGramBlock + warp * 32;  // warp-uniform trip count: the fp32 flush stays convergent
+  int since_flush = 0;
+  for (int64_t base = first; base < n; base += stride) {
+    const int64_t s = base + lane;
+    if (s < n) {
+      if constexpr (PATH == PATH_GENERIC) {
+        T rq[RBM_MAX_JOINTS], rqd[RBM_MAX_JOINTS], rqdd[RBM_MAX_JOINTS], rt[RBM_MAX_JOINTS], t0[RBM_MAX_JOINTS];
+        for (int j = 0; j < nj; ++j) {
+          rq[j] = __ldg(q + j * ld + s); rqd[j] = __ldg(qd + j * ld + s); rqdd[j] = __ldg(qdd + j * ld + s); rt[j] = __ldg(tau + j * ld + s);
+        }
+        payload_generic<T>(sp, nj, rq, rqd, rqdd, t0, [&](int i, const T (&phi)[10]) { payload_accumulate_row(acc, phi, rt[i] - t0[i], false); });
+      } else {
+        using D = std::conditional_t<PATH == PATH_SEQ_ISO, SeqIso, SeqRigid>;
+        T rq[6], rqd[6], rqdd[6], rt[6], t0[6];
+        payload_load_fast(q, qd, qdd, s, ld, rq, rqd, rqdd);
+#pragma unroll
+        for (int j = 0; j < 6; ++j) rt[j] = __ldg(tau + j * ld + s);
+        payload_fast<T, D, SEN_DIAG>(P, rq, rqd, rqdd, t0,
+                                     [&](int j, const T (&phi)[10]) { payload_accumulate_row(acc, phi, rt[j] - t0[j], fast_prismatic<D>(j)); });
+      }
+    }
+    if constexpr (sizeof(T) == 4) {
+      if (++since_flush == kFlush) {
+        since_flush = 0;
+        gram_flush_f32(acc, red[warp], lane);
+      }
+    }
+  }
+  gram_block_epilogue<T>(acc, red, partials);
+}
+
+// partials [nblocks][66] -> pack [112] = [Phi^T Phi (100, row-major) | Phi^T r (10) | r^T r | n]
+__global__ void __launch_bounds__(128) k_payload_finalize(const double* __restrict__ partials, int nblocks, double n_samples, double* __restrict__ pack) {
+  gram_finalize<kPayAcc>(partials, nblocks, n_samples, pack, [](const double* tot, int t) { return payload_pack_entry(tot, t); });
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -569,11 +692,49 @@ int launch_regressor_gram(const rbm_model* m, const T* q, const T* qd, const T* 
   return RBM_OK;
 }
 
+template <class T>
+int launch_payload_regressor(const rbm_model* m, const T* q, const T* qd, const T* qdd, T* Phi, T* tau0, int64_t n, int64_t ld, cudaStream_t st) {
+  if (n == 0) return RBM_OK;
+  const unsigned grid = (unsigned)((n + kRowsBlock - 1) / kRowsBlock);
+  const int np = generic_param_count(m->nj);
+  const FastParams<T>& P = ModelView<T>::fast(m);
+  const T* gp = ModelView<T>::generic(m);
+  if (m->path == PATH_SEQ_ISO) k_payload_regressor<T, PATH_SEQ_ISO><<<grid, kRowsBlock, 0, st>>>(P, gp, m->nj, np, q, qd, qdd, Phi, tau0, n, ld);
+  else if (m->path == PATH_SEQ_RIGID) k_payload_regressor<T, PATH_SEQ_RIGID><<<grid, kRowsBlock, 0, st>>>(P, gp, m->nj, np, q, qd, qdd, Phi, tau0, n, ld);
+  else k_payload_regressor<T, PATH_GENERIC><<<grid, kRowsBlock, sizeof(T) * np, st>>>(P, gp, m->nj, np, q, qd, qdd, Phi, tau0, n, ld);
+  RBM_CUDA_TRY(cudaGetLastError());
+  return RBM_OK;
+}
+
+// one 256-thread CTA per SM (the 66 accumulators and the kinematics do not fit two): partials within rbm_gram_workspace_bytes
+template <class T>
+int launch_payload_gram(const rbm_model* m, const T* q, const T* qd, const T* qdd, const T* tau, double* pack, double* partials, int64_t n, int64_t ld,
+                        cudaStream_t st) {
+  const int grid = gram_grid(m, n, 1);
+  if (n > 0) {
+    const int np = generic_param_count(m->nj);
+    const FastParams<T>& P = ModelView<T>::fast(m);
+    const T* gp = ModelView<T>::generic(m);
+    const bool diag = P.sen_diag != T(0);
+#define RBM_PAYLOAD_GRAM(PATH, DIAG, SMEM) k_payload_gram<T, PATH, DIAG><<<grid, kGramBlock, SMEM, st>>>(P, gp, m->nj, np, q, qd, qdd, tau, partials, n, ld)
+    if (m->path == PATH_SEQ_ISO) diag ? RBM_PAYLOAD_GRAM(PATH_SEQ_ISO, true, 0) : RBM_PAYLOAD_GRAM(PATH_SEQ_ISO, false, 0);
+    else if (m->path == PATH_SEQ_RIGID) diag ? RBM_PAYLOAD_GRAM(PATH_SEQ_RIGID, true, 0) : RBM_PAYLOAD_GRAM(PATH_SEQ_RIGID, false, 0);
+    else RBM_PAYLOAD_GRAM(PATH_GENERIC, false, sizeof(T) * np);
+#undef RBM_PAYLOAD_GRAM
+    RBM_CUDA_TRY(cudaGetLastError());
+  }
+  k_payload_finalize<<<1, 128, 0, st>>>(partials, n > 0 ? grid : 0, (double)n, pack);
+  RBM_CUDA_TRY(cudaGetLastError());
+  return RBM_OK;
+}
+
 #define RBM_INST(T)                                                                                                                        \
   template int launch_regressor_rows<T>(const T*, const T*, T*, int64_t, cudaStream_t);                                                    \
   template int launch_sensor_twists<T>(const double*, const T*, const T*, T*, T*, int64_t, cudaStream_t);                                  \
   template int launch_regressor_from_traj<T>(const rbm_model*, const T*, const T*, const T*, T*, T*, T*, const T*, T*, int64_t, int64_t, cudaStream_t); \
-  template int launch_regressor_gram<T>(const rbm_model*, const T*, const T*, const T*, const T*, double*, double*, int64_t, int64_t, cudaStream_t);
+  template int launch_regressor_gram<T>(const rbm_model*, const T*, const T*, const T*, const T*, double*, double*, int64_t, int64_t, cudaStream_t); \
+  template int launch_payload_regressor<T>(const rbm_model*, const T*, const T*, const T*, T*, T*, int64_t, int64_t, cudaStream_t);                  \
+  template int launch_payload_gram<T>(const rbm_model*, const T*, const T*, const T*, const T*, double*, double*, int64_t, int64_t, cudaStream_t);
 RBM_INST(double)
 RBM_INST(float)
 

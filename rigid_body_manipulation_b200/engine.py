@@ -363,14 +363,52 @@ class Model:
             pack = torch.empty(112, dtype=torch.float64, device=q.device)
         elif pack.shape != (112,) or pack.dtype != torch.float64:
             raise ValueError("pack must be a float64 tensor of 112 elements")
-        ws_bytes = int(self._lib.rbm_gram_workspace_bytes(self._h, n))
-        ws = getattr(self, "_gram_ws", None)
-        if ws is None or ws.numel() * 8 < ws_bytes:
-            ws = self._gram_ws = torch.empty(max(1, ws_bytes // 8), dtype=torch.float64, device=self.device)
+        ws = self._gram_workspace(n)
         fn = self._lib.rbm_regressor_gram_f64 if dt == torch.float64 else self._lib.rbm_regressor_gram_f32
         with torch.cuda.device(self.device):
             rc = fn(self._h, _ptr(q), _ptr(qd), _ptr(qdd), _ptr(f), _ptr(pack), _ptr(ws), ws.numel() * 8, n, n, self._stream())
         _lib.check(rc, "rbm_regressor_gram")
+        return pack
+
+    def _gram_workspace(self, n):
+        """Device scratch of the Gram kernels (rbm_gram_workspace_bytes), cached on the model and grown on demand."""
+        ws_bytes = int(self._lib.rbm_gram_workspace_bytes(self._h, n))
+        ws = getattr(self, "_gram_ws", None)
+        if ws is None or ws.numel() * 8 < ws_bytes:
+            ws = self._gram_ws = torch.empty(max(1, ws_bytes // 8), dtype=torch.float64, device=self.device)
+        return ws
+
+    # ---- payload identification from joint torques -------------------------------------------------------
+    def payload_regressor(self, q, qd, qdd, want_rows=True, want_tau0=False):
+        """Joint-torque payload regressor of this model (the robot WITHOUT the payload): tau = tau0 + Phi phi with phi the payload's 10
+        parameters in the sensor frame (pose_sen_llj), as in `regressor_from_traj`.  Returns a dict with Phi (n, nj, 10) and tau0
+        (nj, n), each None unless asked for."""
+        n, dt = self._check_soa(q, qd, qdd)
+        kw = dict(dtype=dt, device=q.device)
+        Phi = torch.empty((n, self.nj, 10), **kw) if want_rows else None
+        tau0 = torch.empty((self.nj, n), **kw) if want_tau0 else None
+        fn = self._lib.rbm_payload_regressor_f64 if dt == torch.float64 else self._lib.rbm_payload_regressor_f32
+        with torch.cuda.device(self.device):
+            rc = fn(self._h, _ptr(q), _ptr(qd), _ptr(qdd), _ptr(Phi), _ptr(tau0), n, n, self._stream())
+        _lib.check(rc, "rbm_payload_regressor")
+        return dict(Phi=Phi, tau0=tau0)
+
+    def payload_gram(self, q, qd, qdd, tau, pack=None):
+        """Normal equations of the joint-torque route from measured torques tau (nj, n): the 112-double device pack
+        [Phi^T Phi | Phi^T r | r^T r | n] with r = tau - tau0, solved like an F/T pack by identification.solve."""
+        n, dt = self._check_soa(q, qd, qdd)
+        self._check_dev(tau, pack)
+        if tau.shape != (self.nj, n) or tau.dtype != dt:
+            raise ValueError(f"tau must have shape ({self.nj}, n) and the dtype of q")
+        if pack is None:
+            pack = torch.empty(112, dtype=torch.float64, device=q.device)
+        elif pack.shape != (112,) or pack.dtype != torch.float64:
+            raise ValueError("pack must be a float64 tensor of 112 elements")
+        ws = self._gram_workspace(n)
+        fn = self._lib.rbm_payload_gram_f64 if dt == torch.float64 else self._lib.rbm_payload_gram_f32
+        with torch.cuda.device(self.device):
+            rc = fn(self._h, _ptr(q), _ptr(qd), _ptr(qdd), _ptr(tau), _ptr(pack), _ptr(ws), ws.numel() * 8, n, n, self._stream())
+        _lib.check(rc, "rbm_payload_gram")
         return pack
 
     def regressor_gram_grouped(self, q, qd, qdd, f):

@@ -5,6 +5,11 @@ that matrix is 48 GB, so the device accumulates the normal equations instead (rb
 the 112-double pack, and the 10x10 system is solved here in float64 on the host (once per solve, O(1e3) flops).
 
 pack layout: [Y^T Y (100, row-major) | Y^T f (10) | f^T f | n_samples].
+
+The same parameters can be identified from joint torques instead of the wrist sensor (Model.payload_gram, rbm_payload_gram_*): on
+the model without the payload, tau = tau0 + Phi phi, and the pack [Phi^T Phi | Phi^T r | r^T r | n] of r = tau - tau0 has exactly
+this layout.  `solve`, `solve_many` and distributed.allreduce_gram therefore apply unchanged to either route, and the packs of the
+two routes may be summed into one estimate.
 Parameter order: [m, m cx, m cy, m cz, Ixx, Iyy, Izz, Ixy, Iyz, Izx] about the sensor-frame origin
 (reference dynamics.py:225-230, loggers.py:133).
 """
