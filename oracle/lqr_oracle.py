@@ -27,11 +27,20 @@ import numpy as np
 from . import rnea_vec as rv
 
 
+def tip_kw(consts):
+    """The optional tip load of `consts` ("wrench_tip", "pose_tip_Rt", as in rbm_model_create) as keyword arguments of
+    rnea_vec.inverse_batched; empty when the model has none."""
+    return {k: consts[k] for k in ("wrench_tip", "pose_tip_Rt") if consts.get(k) is not None}
+
+
 def _id(consts, q, qd, qdd, gravity=True):
+    """Inverse dynamics; gravity=False switches off the base motion AND the tip wrench, so that ID(q, 0, e_j) is column j of M.
+    The tip wrench is a constant external load: it belongs to the bias h, never to M."""
     traj = np.stack([q, qd, qdd], axis=1)
     dtw0 = consts["dtwist_0"] if gravity else np.zeros(6)
     tw0 = consts["twist_0"] if gravity else np.zeros(6)
-    return rv.inverse_batched(traj, consts["hposes_Rt"], consts["simats"], consts["uscrews"], tw0, dtw0)["tau"]
+    kw = tip_kw(consts) if gravity else {}
+    return rv.inverse_batched(traj, consts["hposes_Rt"], consts["simats"], consts["uscrews"], tw0, dtw0, **kw)["tau"]
 
 
 def mass_matrix(consts, q):

@@ -43,7 +43,8 @@ def inertia_to_phi(G):
 
 
 def _sensor_state(consts, pose_sen_Rt, q, qd, qacc):
-    out = rv.inverse_batched(np.stack([q, qd, qacc])[None], consts["hposes_Rt"], consts["simats"], consts["uscrews"], consts["twist_0"], consts["dtwist_0"])
+    out = rv.inverse_batched(np.stack([q, qd, qacc])[None], consts["hposes_Rt"], consts["simats"], consts["uscrews"], consts["twist_0"], consts["dtwist_0"],
+                             **lo.tip_kw(consts))
     return rv.sensor_frame_twists_batched(pose_sen_Rt, out["twists"][:, -1], out["dtwists"][:, -1])
 
 
@@ -69,7 +70,8 @@ def closed_loop_replay(consts, pose_sen_Rt, G_s, plan_traj, K, q0, qd0=None, dt=
     time = 0.0
     qacc = lo.forward_dynamics(consts, q[None], qd[None], np.zeros((1, nj)))[0]
     wrench = _ft_reading(G_s, *_sensor_state(consts, pose_sen_Rt, q, qd, qacc))
-    tgt_ctrl_all = rv.inverse_batched(plan_traj, consts["hposes_Rt"], consts["simats"], consts["uscrews"], consts["twist_0"], consts["dtwist_0"])["tau"]
+    tgt_ctrl_all = rv.inverse_batched(plan_traj, consts["hposes_Rt"], consts["simats"], consts["uscrews"], consts["twist_0"], consts["dtwist_0"],
+                                      **lo.tip_kw(consts))["tau"]
     log = dict(step=[], time=[], tgt=[], act=[], twist_sen=[], dtwist_sen=[], wrench=[], regressor=[], ctrl=[])
     frame_count = 0
     for step in range(n_steps):
